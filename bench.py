@@ -267,7 +267,14 @@ def main():
                          "(comma list; lock-step groups of up to 16 share a weight sweep); 0 = skip")
     ap.add_argument("--serving-requests", type=int, default=32, dest="serving_requests",
                     help="extra leg at N=1: this many requests through serving.BatchScheduler (16 concurrent); 0 = skip")
+    ap.add_argument("--dump-outputs", default=None, dest="dump_outputs", metavar="DIR",
+                    help="after the timed steps, write what the last timed step of the headline leg returned as DIR/<name>.npy "
+                         "(float32: codes [frames, 16] and the streamed audio), so two builds can be compared output for output")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs applies to the b200 arm")
     args.warmup = max(args.warmup, 3) if args.impl == "b200" else args.warmup
     if args.impl == "reference":
         return run_reference(args)
@@ -282,6 +289,8 @@ def main():
     if not torch.cuda.is_available():
         raise SystemExit("bench.py needs a CUDA device (the engine has no CPU path); use --impl reference for the CPU arm")
     torch.cuda.set_device(local)
+    # every utterance draws its sampling seed from torch's RNG (generate._fresh_seed): seeded, the same arguments sample the same ids
+    torch.manual_seed(0)
     if world > 1:
         dist.init_process_group("nccl", device_id=torch.device("cuda", local))
 
@@ -316,14 +325,24 @@ def main():
                                                                         non_streaming_mode=True)
     launch_events = []
 
-    def dev_step(events=None):
+    def keep_codes(stream, into):
+        for chunk, timing in stream:
+            into.append(chunk)
+            yield chunk, timing
+
+    def dev_step(events=None, keep=None):
+        """keep: None, or a dict whose "codes" / "audio" lists receive the step's device tensors (references, no copies)."""
         stream = fast_generate_streaming(
             talker=talker, talker_input_embeds=tie, attention_mask=tam, trailing_text_hiddens=tth, tts_pad_embed=tpe,
             config=tconf, predictor_graph=model.predictor_graph, talker_graph=model.talker_graph, chunk_size=args.chunk,
             launch_events=events, **gen_kw)
+        if keep is not None:
+            stream = keep_codes(stream, keep["codes"])
         n = 0
         for audio, sr, _ in model._stream_audio(m, stream, None, args.chunk, to_host=False):
             n += audio.numel()
+            if keep is not None:
+                keep["audio"].append(audio)
         return n / sr
 
     for _ in range(args.warmup):
@@ -349,8 +368,9 @@ def main():
     ev0, ev1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     ev0.record()
     audio_s = 0.0
-    for _ in range(args.steps):
-        audio_s += dev_step(launch_events)
+    last = {"codes": [], "audio": []}
+    for i in range(args.steps):
+        audio_s += dev_step(launch_events, last if args.dump_outputs and i == args.steps - 1 else None)
     ev1.record()
     barrier()
     launches = eng.launch_count + codec.launch_count - l0
@@ -368,6 +388,12 @@ def main():
     clk = clocks.stop()
 
     (dev_ms, e2e_ms), (audio_all, e2e_audio_all) = aggregate_over_ranks([dev_ms, e2e_s * 1000.0], [audio_s, e2e_audio_s], dev, world)
+
+    if args.dump_outputs and rank == 0:
+        # codes [frames, 16] and audio [frames * 1920]: at most 16 MB in all, since max_seq_len 2048 bounds the frames
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        for name, parts in last.items():
+            np.save(os.path.join(args.dump_outputs, f"{name}.npy"), torch.cat(parts).float().cpu().numpy())
 
     if rank == 0:
         pb = param_bytes(model.model.cfg)

@@ -71,3 +71,15 @@ def test_reference_arm_prints_the_contract_line_on_rank_0_only():
     assert "workload" in d["config"] and "model" not in d["config"] and d["config"]["reference_sample"]["frames_per_step"] == 8
     r1 = subprocess.run(cmd, env=dict(env, RANK="1", WORLD_SIZE="2"), capture_output=True, text=True, timeout=300)
     assert r1.returncode == 0 and r1.stdout.strip() == ""
+
+
+def test_zero_steps_and_a_dump_from_the_cpu_arm_are_refused(tmp_path):
+    """--steps sets the number of timed steps, so fewer than one is an error; --dump-outputs writes the B200 arm's outputs and is
+    refused for the CPU arm instead of being ignored.  Nothing is written."""
+    import subprocess
+
+    bench = os.path.join(ROOT, "bench.py")
+    for args in (["--steps", "0"], ["--impl", "reference", "--dump-outputs", str(tmp_path / "d")]):
+        r = subprocess.run([sys.executable, bench] + args, capture_output=True, text=True, timeout=120)
+        assert r.returncode == 2 and "error" in r.stderr, (args, r.stderr[-500:])
+    assert not (tmp_path / "d").exists()
