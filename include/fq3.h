@@ -101,8 +101,24 @@ int fq3_num_sms(const fq3_engine* e);
 int64_t fq3_launch_count(const fq3_engine* e);
 
 /* ---- per-utterance set-up ------------------------------------------------------------------ */
-/* TalkerGraph.reset (talker_graph.py:149-151): forget KV, history, frame count of one stream. */
+/* TalkerGraph.reset (talker_graph.py:149-151): forget KV, history, frame count of one stream.  Also clears the stream's
+ * sampling policy record (fq3_set_stream_policy). */
 int fq3_reset_stream(fq3_engine* e, int stream_idx, void* stream);
+/* Serving (no counterpart in the reference): a stream's own sampling policy, so that requests with different sampling
+ * arguments share one lock-step launch.  While a stream has a record, fq3_prefill / fq3_prefill_tail / fq3_prefill_head
+ * (first-token sample) and fq3_decode_frames (any n_streams, both frame programs, every lock-step group) sample that stream
+ * with the record instead of the `policy` argument: do_sample, top_k, top_p, temperature, repetition_penalty, min_new_tokens
+ * (both EOS-suppression rules), suppress_tail and seed for the first codebook; for codebooks 1..15 the seed only (their
+ * arguments stay the launch's fq3_subpolicy, frozen at capture time in the reference, predictor_graph.py:34-50).  The Philox
+ * key of such a stream is seed ^ K * 1 whatever its slot — the key slot 0 gets under a launch-wide policy with the same seed —
+ * so its draws depend only on its own seed and draw counter, and it draws exactly what a single-stream run in slot 0 with a
+ * launch-wide policy of the same values draws.  Streams without a record sample exactly as before.  fq3_talker_step,
+ * fq3_predictor_run and fq3_sample take their arguments explicitly and ignore the record.
+ * Stream-ordered (the record is written by a kernel on `stream`; `policy` may be freed when the call returns).
+ * policy == NULL clears the record.  The record survives the reset a prefill runs internally; fq3_reset_stream clears it.
+ * -FQ3_E_INVALID for an index out of range, top_k < 0, top_p outside (0, 1], temperature <= 0 with do_sample,
+ * repetition_penalty <= 0, suppress_tail outside [0, V_t]. */
+int fq3_set_stream_policy(fq3_engine* e, int stream_idx, const fq3_policy* policy, void* stream);
 /* Serving (no counterpart in the reference, whose servers hold one lock around a bs = 1 model: examples/openai_server.py:71,181):
  * take one stream out of the lock-step frame loop — it idles (status.done = 3) in every later fq3_decode_frames until it is
  * reset and prefilled again.  A scheduler retires the slot of a finished / cancelled / length-capped request so that the

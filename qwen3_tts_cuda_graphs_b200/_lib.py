@@ -60,6 +60,7 @@ SYMBOLS = {
     "fq3_launch_count": (C.c_int64, [_P]),
     "fq3_reset_stream": (C.c_int, [_P, C.c_int, _P]),
     "fq3_retire_stream": (C.c_int, [_P, C.c_int, _P]),
+    "fq3_set_stream_policy": (C.c_int, [_P, C.c_int, C.POINTER(Policy), _P]),
     "fq3_set_generation_state": (C.c_int, [_P, C.c_int, C.c_int, C.c_int, _P]),
     "fq3_set_text_conditioning": (C.c_int, [_P, C.c_int, _P, C.c_int, _P, _P]),
     "fq3_import_kv": (C.c_int, [_P, C.c_int, C.c_int, _P, _P, C.c_int, _P]),

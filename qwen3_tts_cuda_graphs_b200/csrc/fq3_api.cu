@@ -52,6 +52,9 @@ struct fq3_engine {
   size_t buf_bytes[kNumBufs] = {};
   StackRt rt[2]{};
   StreamState* d_st = nullptr;
+  StreamPolicy* d_spol = nullptr;  // [max_streams] per-stream sampling policies (fq3_set_stream_policy), zeroed = none
+  std::vector<uint8_t> spol_on;    // host mirror of the records' `on` flags, in call order: a launch none of whose streams has a
+                                   // record gets no record pointer, so its samplers issue no extra load on the critical path
   std::vector<StreamState> h_st;
   LLWord* attn_part = nullptr;
   size_t attn_part_bytes = 0;
@@ -635,7 +638,9 @@ static int create_impl(const fq3_model_desc* desc, fq3_engine* e) {
   // --- per-stream state ---
   e->h_st.resize(B);
   e->in_wpin.assign(B, 0);
+  e->spol_on.assign(B, 0);
   if (dalloc(e, &e->d_st, B)) return -FQ3_E_CUDA;
+  if (dalloc(e, &e->d_spol, B)) return -FQ3_E_CUDA;
   for (int b = 0; b < B; ++b) {
     StreamState& s = e->h_st[b];
     memset(&s, 0, sizeof s);
@@ -728,9 +733,17 @@ static int check_stream(fq3_engine* e, int idx) {
   return 0;
 }
 
+// LaunchParams::spol of a launch over streams [s0, s0 + n): the records when one of them has one, else null
+static const StreamPolicy* spol_for(const fq3_engine* e, int s0, int n) {
+  for (int i = s0; i < s0 + n; ++i)
+    if (e->spol_on[i]) return e->d_spol;
+  return nullptr;
+}
+
 int fq3_reset_stream(fq3_engine* e, int idx, void* stream) {
   if (int r = check_stream(e, idx)) return r;
-  fq3_reset_stream_kernel<<<1, 256, 0, (cudaStream_t)stream>>>(e->d_st + idx, e->tk.d.vocab);
+  fq3_reset_stream_kernel<<<1, 256, 0, (cudaStream_t)stream>>>(e->d_st + idx, e->tk.d.vocab, e->d_spol + idx);
+  e->spol_on[idx] = 0;
   e->launches += 1;
   CK(cudaGetLastError());
   return 0;
@@ -739,6 +752,24 @@ int fq3_reset_stream(fq3_engine* e, int idx, void* stream) {
 int fq3_retire_stream(fq3_engine* e, int idx, void* stream) {
   if (int r = check_stream(e, idx)) return r;
   fq3_set_state_kernel<<<1, 32, 0, (cudaStream_t)stream>>>(e->d_st + idx, 0, 0, 0, 32, 0, 0, 0);
+  e->launches += 1;
+  CK(cudaGetLastError());
+  return 0;
+}
+
+int fq3_set_stream_policy(fq3_engine* e, int idx, const fq3_policy* policy, void* stream) {
+  if (int r = check_stream(e, idx)) return r;
+  Policy pol{};
+  if (policy) {
+    if (policy->top_k < 0) return fail(FQ3_E_INVALID, "top_k < 0");
+    if (!(policy->top_p > 0.0f && policy->top_p <= 1.0f)) return fail(FQ3_E_INVALID, "top_p outside (0, 1]");
+    if (policy->do_sample && !(policy->temperature > 0.0f)) return fail(FQ3_E_INVALID, "temperature <= 0 with do_sample");
+    if (!(policy->repetition_penalty > 0.0f)) return fail(FQ3_E_INVALID, "repetition_penalty <= 0");
+    if (policy->suppress_tail < 0 || policy->suppress_tail > e->tk.d.vocab) return fail(FQ3_E_INVALID, "suppress_tail outside [0, V]");
+    pol = to_policy(policy);
+  }
+  fq3_set_stream_policy_kernel<<<1, 32, 0, (cudaStream_t)stream>>>(e->d_spol + idx, policy ? 1 : 0, pol);
+  e->spol_on[idx] = policy ? 1 : 0;
   e->launches += 1;
   CK(cudaGetLastError());
   return 0;
@@ -832,7 +863,7 @@ static int prefill_impl(fq3_engine* e, int idx, const void* embeds_from_start, i
   const int Ht = e->tk.d.hidden;
   const int Mmax = prefill_rows(e);
   if (int r = reserve_epochs(e, (uint64_t)((T - start + Mmax - 1) / Mmax) * (uint64_t)(e->n_prefill_ph + 2), s)) return r;
-  fq3_reset_stream_kernel<<<1, 256, 0, s>>>(e->d_st + idx, e->tk.d.vocab);
+  fq3_reset_stream_kernel<<<1, 256, 0, s>>>(e->d_st + idx, e->tk.d.vocab, nullptr);  // the policy record survives
   fq3_set_state_kernel<<<1, 32, 0, s>>>(e->d_st + idx, 0, 0, 0, 2, n_left_pad, -n_left_pad, 0);
   e->launches += 2;
   for (int c0 = start; c0 < T; c0 += Mmax) {
@@ -848,6 +879,7 @@ static int prefill_impl(fq3_engine* e, int idx, const void* embeds_from_start, i
     p.stream0 = idx;
     p.pf_pos0 = c0; p.pf_n_pad = n_left_pad; p.pf_rope_delta = -n_left_pad; p.pf_final = final;
     p.pol = to_policy(policy);
+    p.spol = spol_for(e, idx, 1);
     if (int r = launch(e, p, e->h_prefill.data(), s)) return r;
   }
   fq3_set_state_kernel<<<1, 32, 0, s>>>(e->d_st + idx, 0, T, 0, 8, 0, 0, 0);
@@ -882,7 +914,7 @@ int fq3_prefill_head(fq3_engine* e, int idx, const void* last_hidden, int T, con
   cudaStream_t s = (cudaStream_t)stream;
   const int Ht = e->tk.d.hidden;
   if (int r = reserve_epochs(e, 4, s)) return r;
-  fq3_reset_stream_kernel<<<1, 256, 0, s>>>(e->d_st + idx, e->tk.d.vocab);
+  fq3_reset_stream_kernel<<<1, 256, 0, s>>>(e->d_st + idx, e->tk.d.vocab, nullptr);  // the policy record survives
   fq3_set_state_kernel<<<1, 32, 0, s>>>(e->d_st + idx, 0, 0, 0, 2, 0, 0, 0);
   e->launches += 2;
   if (int r = pack_ll(e, BUF_TX, 0, last_hidden, Ht, 1, Ht, s)) return r;
@@ -896,6 +928,7 @@ int fq3_prefill_head(fq3_engine* e, int idx, const void* last_hidden, int T, con
   p.stream0 = idx;
   p.pf_pos0 = T - 1; p.pf_n_pad = 0; p.pf_rope_delta = 0; p.pf_final = 1;
   p.pol = to_policy(policy);
+  p.spol = spol_for(e, idx, 1);
   if (int r = launch(e, p, e->h_prefill.data() + (e->n_prefill_ph - 2), s)) return r;
   fq3_set_state_kernel<<<1, 32, 0, s>>>(e->d_st + idx, 0, T, 0, 8, 0, 0, 0);
   e->in_wpin[idx] = 0;
@@ -1030,6 +1063,7 @@ int fq3_decode_frames(fq3_engine* e, int n_streams, int n_frames, const fq3_poli
       p.stream0 = s0;
       p.n_iters = n_frames;
       p.pol = to_policy(policy);
+      p.spol = spol_for(e, s0, n);
       p.sub = to_sub(sub);
       if (int r = launch(e, p, e->h_wide.data(), (cudaStream_t)stream)) return r;
     }
@@ -1045,6 +1079,7 @@ int fq3_decode_frames(fq3_engine* e, int n_streams, int n_frames, const fq3_poli
   p.n_rows = n_streams;
   p.n_iters = n_frames;
   p.pol = to_policy(policy);
+  p.spol = spol_for(e, 0, n_streams);
   p.sub = to_sub(sub);
   return launch(e, p, e->h_frames.data(), (cudaStream_t)stream);
 }

@@ -195,6 +195,13 @@ struct SubPolicy {
   int do_sample, top_k;
   float top_p, temperature;
 };
+// A stream's own sampling policy (fq3_set_stream_policy), one per stream in device memory.  on != 0: the stream's talker /
+// prefill sampler takes pol instead of LaunchParams::pol and its predictor sampler takes pol.seed; the Philox key is then
+// pol.seed ^ K * 1 whatever the slot, so the draws depend on the stream's seed and draw counter alone.
+struct StreamPolicy {
+  int on;
+  Policy pol;
+};
 
 enum Mode : int { MODE_FRAMES = 0, MODE_TALKER_STEP = 1, MODE_PREDICTOR = 2, MODE_PREFILL = 3, MODE_LINEAR = 4 };
 
@@ -219,6 +226,7 @@ struct LaunchParams {
   StreamState* st;
   Policy pol;
   SubPolicy sub;
+  const StreamPolicy* spol;  // [max_streams] per-stream policies; null when no stream of the launch has one, or the launch takes its policy explicitly
   LLWord* attn_part;  // split-attention partials as fp32 LL words [row][q head][split][kPartStride]
   int* err;  // mapped host memory: [0]=code [1]=cta [2]=phase [3]=detail
   // model constants used by the sampling phases

@@ -2654,10 +2654,13 @@ __device__ __forceinline__ void sample_phase(const Phase& ph, const LaunchParams
           p.pred_logits_all[(size_t)i * Vp + 2 * v + 1] = bf_hi(pay);
         }
       }
+      // codebooks 1..15 keep the launch's SubPolicy; a stream with its own policy keys the draws with its own seed (fq3_common.cuh)
+      const bool own = p.spol != nullptr && __ldcg(&p.spol[slot].on) != 0;
+      const unsigned long long seed = own ? __ldcg(&p.spol[slot].pol.seed) : p.pol.seed;
       SampleArgs a;
       a.V = Vp; a.do_sample = p.sub.do_sample; a.top_k = p.sub.top_k; a.top_p = p.sub.top_p;
       a.temperature = p.sub.temperature; a.rep_pen = 1.0f; a.seen = nullptr; a.suppress_start = Vp; a.eos = -1;
-      a.suppress_eos = 0; a.round_bf16 = 1; a.seed = p.pol.seed ^ (0x9E3779B97F4A7C15ull * (unsigned long long)(slot + 1));
+      a.suppress_eos = 0; a.round_bf16 = 1; a.seed = seed ^ (0x9E3779B97F4A7C15ull * (unsigned long long)(own ? 1 : slot + 1));
       a.draw = __ldcg(&st->draws) + (unsigned long long)(i + 1);
       a.next_emb = p.pred_embeds[i]; a.emb_row_bytes = Ht * 2;
       const int tok = sample_ll(lg, ep_in, p, pidx, a, sm.scratch);
@@ -2711,14 +2714,25 @@ __device__ __forceinline__ void sample_phase(const Phase& ph, const LaunchParams
       const LLWord* lg = lgbuf + (size_t)b * p.ld[BUF_LOGITS];
       const int nfr = __ldcg(&st->n_frames);
       const int done_now = (ph.skind == SMP_PREFILL) ? 0 : __ldcg(&st->done);  // includes this frame's cache-bound stop
+      // the stream's own policy when it has one (fq3_set_stream_policy), else the launch's; read once into registers
+      const bool own = p.spol != nullptr && __ldcg(&p.spol[slot].on) != 0;
+      Policy pol;
+      if (own) {
+        const Policy* sp = &p.spol[slot].pol;
+        pol.do_sample = __ldcg(&sp->do_sample); pol.top_k = __ldcg(&sp->top_k); pol.top_p = __ldcg(&sp->top_p);
+        pol.temperature = __ldcg(&sp->temperature); pol.rep_pen = __ldcg(&sp->rep_pen);
+        pol.min_new_tokens = __ldcg(&sp->min_new_tokens); pol.suppress_tail = __ldcg(&sp->suppress_tail); pol.seed = __ldcg(&sp->seed);
+      } else {
+        pol = p.pol;
+      }
       SampleArgs a;
-      a.V = Vt; a.do_sample = p.pol.do_sample; a.top_k = p.pol.top_k; a.top_p = p.pol.top_p;
-      a.temperature = p.pol.temperature; a.rep_pen = p.pol.rep_pen;
+      a.V = Vt; a.do_sample = pol.do_sample; a.top_k = pol.top_k; a.top_p = pol.top_p;
+      a.temperature = pol.temperature; a.rep_pen = pol.rep_pen;
       a.seen = (ph.skind == SMP_TALKER && nfr > 0) ? st->seen : nullptr;
-      a.suppress_start = max(0, Vt - p.pol.suppress_tail); a.eos = p.eos_id;
-      a.suppress_eos = (ph.skind == SMP_PREFILL) ? (p.pol.min_new_tokens > 0) : (nfr < p.pol.min_new_tokens);
+      a.suppress_start = max(0, Vt - pol.suppress_tail); a.eos = p.eos_id;
+      a.suppress_eos = (ph.skind == SMP_PREFILL) ? (pol.min_new_tokens > 0) : (nfr < pol.min_new_tokens);
       a.round_bf16 = 1;
-      a.seed = p.pol.seed ^ (0x9E3779B97F4A7C15ull * (unsigned long long)(slot + 1));
+      a.seed = pol.seed ^ (0x9E3779B97F4A7C15ull * (unsigned long long)(own ? 1 : slot + 1));
       a.draw = __ldcg(&st->draws);
       a.next_emb = p.codec_embed; a.emb_row_bytes = Ht * 2;
       int tok = sample_ll(lg, ep_in, p, pidx, a, sm.scratch);
@@ -3032,12 +3046,22 @@ __global__ void fq3_ctl_clear_epochs_kernel(StreamState* st, int n) {
   for (int i = threadIdx.x; i < n * 4; i += blockDim.x) st[i >> 2].ctl[i & 3].y = 0u;
 }
 
-__global__ void fq3_reset_stream_kernel(StreamState* st, int V) {
+// spol: the stream's policy record to clear as well (fq3_reset_stream), null where it survives (the reset inside a prefill)
+__global__ void fq3_reset_stream_kernel(StreamState* st, int V, StreamPolicy* spol) {
   for (int i = threadIdx.x; i < V; i += blockDim.x) st->seen[i] = 0;
   if (threadIdx.x == 0) {
     st->token = 0; st->position = 0; st->gen_step = 0; st->n_frames = 0; st->done = 0; st->n_pad = 0;
     st->rope_delta = 0; st->draws = 0ull;  // text conditioning (n_trailing) is set separately and survives a reset
     for (int i = 0; i < 32; ++i) st->cur_codes[i] = 0;
+    if (spol) spol->on = 0;
+  }
+}
+
+// fq3_set_stream_policy: the policy travels by value, so no host buffer has to outlive the (stream-ordered) call
+__global__ void fq3_set_stream_policy_kernel(StreamPolicy* spol, int on, Policy pol) {
+  if (threadIdx.x == 0) {
+    spol->pol = pol;
+    spol->on = on;
   }
 }
 

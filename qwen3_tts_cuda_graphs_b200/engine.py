@@ -29,6 +29,26 @@ class SamplingPolicy:
     suppress_tail: int = 1024
     seed: int = 0
 
+    def validate(self, vocab: Optional[int] = None) -> "SamplingPolicy":
+        """ValueError for out-of-range sampling values: what fq3_set_stream_policy refuses (fq3.h: top_k < 0, top_p outside
+        (0, 1], temperature <= 0 with do_sample, repetition_penalty <= 0, suppress_tail outside [0, vocab]), a negative
+        min_new_tokens and a seed that does not fit 64 bits."""
+        if int(self.top_k) < 0:
+            raise ValueError(f"top_k must be >= 0, got {self.top_k}")
+        if not 0.0 < float(self.top_p) <= 1.0:
+            raise ValueError(f"top_p must be in (0, 1], got {self.top_p}")
+        if self.do_sample and not float(self.temperature) > 0.0:
+            raise ValueError(f"temperature must be > 0 when sampling, got {self.temperature}")
+        if not float(self.repetition_penalty) > 0.0:
+            raise ValueError(f"repetition_penalty must be > 0, got {self.repetition_penalty}")
+        if int(self.min_new_tokens) < 0:
+            raise ValueError(f"min_new_tokens must be >= 0, got {self.min_new_tokens}")
+        if int(self.suppress_tail) < 0 or (vocab is not None and int(self.suppress_tail) > vocab):
+            raise ValueError(f"suppress_tail must be in [0, {vocab}], got {self.suppress_tail}")
+        if not 0 <= int(self.seed) < 2**64:
+            raise ValueError(f"seed must be in [0, 2**64), got {self.seed}")
+        return self
+
     def c(self) -> _lib.Policy:
         return _lib.Policy(
             int(self.do_sample), int(self.top_k), float(self.top_p), float(self.temperature),
@@ -146,6 +166,12 @@ class Engine:
     def retire_stream(self, idx: int):
         """Take a slot out of the lock-step frame loop until its next reset + prefill (fq3.h: fq3_retire_stream)."""
         _lib.check(self.lib.fq3_retire_stream(self.h, idx, _stream()))
+
+    def set_stream_policy(self, idx: int, policy: Optional[SamplingPolicy]):
+        """A stream's own sampling policy, seed included, used by its prefill and every frame-loop launch instead of the launch's
+        policy (fq3.h: fq3_set_stream_policy); None clears it.  Survives prefill; reset_stream clears it."""
+        pol = None if policy is None else C.byref(policy.c())
+        _lib.check(self.lib.fq3_set_stream_policy(self.h, int(idx), pol, _stream()))
 
     def set_generation_state(self, idx: int, n_left_pad: int, rope_delta: int):
         _lib.check(self.lib.fq3_set_generation_state(self.h, idx, int(n_left_pad), int(rope_delta), _stream()))

@@ -15,7 +15,7 @@ max_seq_len-1 stop) are the ones in SURVEY.md Appendix A1 in both paths.
 from __future__ import annotations
 
 import time
-from typing import Optional, Tuple
+from typing import Optional, Sequence, Tuple
 
 import torch
 
@@ -121,14 +121,24 @@ def fast_generate(
 @torch.inference_mode()
 def fast_generate_batch(talker_graph, predictor_graph, requests, max_new_tokens: int = 2048, min_new_tokens: int = 2,
                         temperature: float = 0.9, top_k: int = 50, top_p: float = 1.0, do_sample: bool = True,
-                        repetition_penalty: float = 1.05, seed: Optional[int] = None):
+                        repetition_penalty: float = 1.05, seed: Optional[int] = None,
+                        policies: Optional[Sequence[SamplingPolicy]] = None):
     """Request-parallel generation (BASELINE configs[3] / [4]; no counterpart in the reference, which is bs = 1): up to
     `engine.max_streams` independent utterances per call; lock-step groups of up to `engine.lockstep_group` (16) of them share
     every weight sweep of the persistent kernel (a stream that hit EOS idles until its group is done; more streams than one
     group run group after group).  `requests` = list of (talker_input_embeds, attention_mask,
     trailing_text_hiddens, tts_pad_embed) as built for fast_generate.  Returns ([codec_ids | None per request], timing).
-    Each stream draws from its own Philox stream (seed ^ slot), so a request's tokens do not depend on its neighbours."""
+    Each stream draws from its own Philox stream (seed ^ slot), so a request's tokens do not depend on its neighbours.
+    `policies`: one SamplingPolicy per request (seed included), set as the stream's own policy for its prefill and frame loop
+    (fq3.h: fq3_set_stream_policy) — requests of different policies share the launches, and each one draws exactly what a
+    single-stream run with that policy and seed draws; the scalar arguments then only make the launch-wide policy no stream uses."""
     eng = talker_graph.engine
+    if policies is not None:
+        policies = list(policies)
+        if len(policies) != len(requests):
+            raise ValueError(f"policies: {len(policies)} for {len(requests)} requests")
+        if not all(isinstance(p, SamplingPolicy) for p in policies):
+            raise ValueError("policies: one SamplingPolicy per request")
     policy = SamplingPolicy(
         do_sample=do_sample, top_k=top_k, top_p=top_p, temperature=temperature, repetition_penalty=repetition_penalty,
         min_new_tokens=min_new_tokens, suppress_tail=1024, seed=_fresh_seed() if seed is None else seed,
@@ -143,15 +153,22 @@ def fast_generate_batch(talker_graph, predictor_graph, requests, max_new_tokens:
     per_call = eng.max_streams if eng.lockstep_group > 4 else min(eng.max_streams, 4)
     for g0 in range(0, len(requests), per_call):
         group = requests[g0:g0 + per_call]
-        for s, (tie, tam, tth, tpe) in enumerate(group):
-            if tie.shape[1] > eng.max_seq_len:
-                raise RuntimeError(
-                    f"Input is too long: prefill has {tie.shape[1]} tokens but max_seq_len={eng.max_seq_len}. "
-                    "Use shorter text or shorter reference audio."
-                )
-            eng.set_text_conditioning(s, tth[0], tpe)
-            eng.prefill(s, tie[0], _left_pads(tam), policy)
-        eng.decode_frames(len(group), min(max_new_tokens, eng.max_frames), policy, sub)
+        try:
+            for s, (tie, tam, tth, tpe) in enumerate(group):
+                if tie.shape[1] > eng.max_seq_len:
+                    raise RuntimeError(
+                        f"Input is too long: prefill has {tie.shape[1]} tokens but max_seq_len={eng.max_seq_len}. "
+                        "Use shorter text or shorter reference audio."
+                    )
+                eng.set_text_conditioning(s, tth[0], tpe)
+                if policies is not None:
+                    eng.set_stream_policy(s, policies[g0 + s])
+                eng.prefill(s, tie[0], _left_pads(tam), policy)
+            eng.decode_frames(len(group), min(max_new_tokens, eng.max_frames), policy, sub)
+        finally:
+            if policies is not None:  # a later caller of these slots (slot 0: the single-stream API) gets the launch's policy again
+                for s in range(len(group)):
+                    eng.set_stream_policy(s, None)
         for s in range(len(group)):
             n = eng.status(s).n_frames
             frames += n

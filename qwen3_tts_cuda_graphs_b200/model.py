@@ -19,11 +19,15 @@ import numpy as np
 import torch
 
 from .base_model import Qwen3TTSBaseModel
+from .engine import SamplingPolicy
 from .predictor_graph import PredictorGraph
 from .sampling import set_default_engine
 from .talker_graph import TalkerGraph
 
 logger = logging.getLogger(__name__)
+
+# sampling arguments one entry of generate_voice_clone_batch(per_request=...) may set
+PER_REQUEST_KEYS = ("temperature", "top_k", "top_p", "do_sample", "repetition_penalty", "min_new_tokens", "seed")
 
 
 class WindowedDecode:
@@ -504,11 +508,29 @@ class FasterQwen3TTS:
     def generate_voice_clone_batch(self, texts: List[str], language: str, ref_audio, ref_text: str, max_new_tokens: int = 2048,
                                    min_new_tokens: int = 2, temperature: float = 0.9, top_k: int = 50, top_p: float = 1.0,
                                    do_sample: bool = True, repetition_penalty: float = 1.05, xvec_only: bool = True,
-                                   non_streaming_mode: bool = True, append_silence: bool = True) -> Tuple[List[np.ndarray], int]:
+                                   non_streaming_mode: bool = True, append_silence: bool = True,
+                                   per_request: Optional[List[dict]] = None) -> Tuple[List[np.ndarray], int]:
         """Several texts in one voice, decoded `max_streams` at a time in lock-step (load the model with
-        `from_pretrained(..., max_streams=4)`).  An extension over the reference's bs = 1 API; returns one waveform per text."""
-        from .generate import fast_generate_batch
+        `from_pretrained(..., max_streams=4)`).  An extension over the reference's bs = 1 API; returns one waveform per text.
+        per_request: one dict of sampling arguments per text (keys of PER_REQUEST_KEYS; a key a dict leaves out takes the scalar
+        argument, a missing `seed` a fresh one): the texts still share every launch, and each one is sampled exactly as
+        generate_voice_clone with those arguments and seed would sample it."""
+        from .generate import _fresh_seed, fast_generate_batch
 
+        policies = None
+        if per_request is not None:
+            if len(per_request) != len(texts):
+                raise ValueError(f"per_request: {len(per_request)} entries for {len(texts)} texts")
+            scalar = dict(temperature=temperature, top_k=top_k, top_p=top_p, do_sample=do_sample,
+                          repetition_penalty=repetition_penalty, min_new_tokens=min_new_tokens)
+            policies = []
+            for d in per_request:
+                unknown = set(d) - set(PER_REQUEST_KEYS)
+                if unknown:
+                    raise ValueError(f"per_request: unknown key(s) {sorted(unknown)}; allowed: {list(PER_REQUEST_KEYS)}")
+                kw = {**scalar, **{k: v for k, v in d.items() if k != "seed"}}
+                seed = d.get("seed")
+                policies.append(SamplingPolicy(suppress_tail=1024, seed=_fresh_seed() if seed is None else int(seed), **kw).validate())
         reqs, metas = [], []
         for text in texts:
             m, talker, config, tie, tam, tth, tpe, ref_codes = self._prepare_generation(
@@ -518,7 +540,7 @@ class FasterQwen3TTS:
             metas.append((m, ref_codes))
         codes, timing = fast_generate_batch(self.talker_graph, self.predictor_graph, reqs, max_new_tokens=max_new_tokens,
                                             min_new_tokens=min_new_tokens, temperature=temperature, top_k=top_k, top_p=top_p,
-                                            do_sample=do_sample, repetition_penalty=repetition_penalty)
+                                            do_sample=do_sample, repetition_penalty=repetition_penalty, policies=policies)
         audio = []
         for c, (m, ref_codes) in zip(codes, metas):
             if c is None:

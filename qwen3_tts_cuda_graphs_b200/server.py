@@ -105,6 +105,7 @@ class SpeechRequest(BaseModel):  # examples/openai_server.py:78-83
     voice: str = "alloy"
     response_format: str = "wav"
     speed: float = 1.0  # accepted, not applied (as in the reference)
+    seed: Optional[int] = None  # sampling seed: the same seed gives the same audio (a server started with --mixed-policies)
 
 
 class BackendUnavailable(RuntimeError):
@@ -157,11 +158,24 @@ def _request_for(voice_cfg: dict, text: str, overrides: Optional[dict] = None) -
         kw.update(kind="voice_design", instruct=voice_cfg["instruct"])
     else:
         raise ValueError("a voice needs ref_audio, speaker or instruct")
-    for k in ("max_new_tokens", "temperature", "top_k", "top_p", "repetition_penalty", "do_sample"):
+    for k in ("max_new_tokens", "temperature", "top_k", "top_p", "repetition_penalty", "do_sample", "seed"):
         if k in voice_cfg:
             kw[k] = voice_cfg[k]
-    kw.update(overrides or {})
-    return TTSRequest(**kw)
+    kw.update({k: v for k, v in (overrides or {}).items() if not (k == "seed" and v is None)})
+    req = TTSRequest(**kw)
+    _check_sampling(req)
+    return req
+
+
+def _check_sampling(req: TTSRequest):
+    """ValueError (HTTP 400) for sampling fields out of range (engine.SamplingPolicy.validate)."""
+    from .engine import SamplingPolicy
+
+    if req.seed is not None and (isinstance(req.seed, bool) or not isinstance(req.seed, int)):
+        raise ValueError(f"seed must be an integer, got {req.seed!r}")
+    SamplingPolicy(do_sample=req.do_sample, top_k=req.top_k, top_p=req.top_p, temperature=req.temperature,
+                   repetition_penalty=req.repetition_penalty, min_new_tokens=req.min_new_tokens,
+                   seed=0 if req.seed is None else req.seed).validate()
 
 
 def create_app(backends: List[object], voices: Dict[str, dict], default_voice: Optional[str] = None, sample_rate: int = 24000,
@@ -222,7 +236,7 @@ def create_app(backends: List[object], voices: Dict[str, dict], default_voice: O
             raise HTTPException(status_code=400, detail=f"response_format {fmt!r} not supported. Use: wav, pcm, mp3")
         segment_cls = mp3_encoder() if fmt == "mp3" else None
         try:
-            handle = disp.submit(_request_for(voice_cfg, req.input))
+            handle = disp.submit(_request_for(voice_cfg, req.input, {"seed": req.seed}))
         except ValueError as e:
             raise HTTPException(status_code=400, detail=str(e))
         except RuntimeError as e:  # BackendUnavailable, or the chosen replica failed between the check and the submit
@@ -247,14 +261,14 @@ def create_app(backends: List[object], voices: Dict[str, dict], default_voice: O
         return StreamingResponse(audio_stream(), media_type=CONTENT_TYPES[fmt], background=BackgroundTask(settle, handle))
 
     async def demo_request(text, language, mode, ref_text, speaker, instruct, xvec_only, temperature, top_k, repetition_penalty,
-                           voice, ref_preset, ref_audio) -> TTSRequest:
+                           voice, ref_preset, ref_audio, seed=None) -> TTSRequest:
         """The demo's form (demo/server.py:332-372, :546-587) -> a request.  Reference audio: an upload, else a configured voice
         (`ref_preset` / `voice`, the demo's presets), else the default voice."""
         if not text.strip():
             raise HTTPException(status_code=400, detail="text is empty")
         if len(text) > MAX_TEXT_CHARS:
             raise HTTPException(status_code=400, detail=f"Text too long ({len(text)} chars). Maximum is {MAX_TEXT_CHARS} characters.")
-        over = dict(language=language, temperature=temperature, top_k=top_k, repetition_penalty=repetition_penalty)
+        over = dict(language=language, temperature=temperature, top_k=top_k, repetition_penalty=repetition_penalty, seed=seed)
         try:
             if mode == "voice_clone":
                 if ref_audio is not None and getattr(ref_audio, "filename", None):
@@ -279,6 +293,8 @@ def create_app(backends: List[object], voices: Dict[str, dict], default_voice: O
     def submit_or_503(req: TTSRequest):
         try:
             return disp.submit(req)
+        except ValueError as e:  # e.g. a seed sent to a server without --mixed-policies
+            raise HTTPException(status_code=400, detail=str(e))
         except RuntimeError as e:
             raise HTTPException(status_code=503, detail=str(e))
 
@@ -330,11 +346,11 @@ def create_app(backends: List[object], voices: Dict[str, dict], default_voice: O
                               ref_text: str = Form(""), speaker: str = Form(""), instruct: str = Form(""),
                               xvec_only: bool = Form(True), chunk_size: int = Form(8), temperature: float = Form(0.9),
                               top_k: int = Form(50), repetition_penalty: float = Form(1.05), voice: str = Form(""),
-                              ref_preset: str = Form(""), ref_audio: UploadFile = File(None)):
+                              ref_preset: str = Form(""), ref_audio: UploadFile = File(None), seed: Optional[int] = Form(None)):
         """The demo's SSE protocol (demo/server.py:332-541).  `chunk_size` is accepted for compatibility: the streaming granularity
         is the scheduler's `chunk_frames` (one launch for all running utterances), set when the server starts."""
         req = await demo_request(text, language, mode, ref_text, speaker, instruct, xvec_only, temperature, top_k, repetition_penalty,
-                                 voice, ref_preset, ref_audio)
+                                 voice, ref_preset, ref_audio, seed)
         ahead = sum(disp.in_flight)
         handle = submit_or_503(req)
         t0 = time.perf_counter()
@@ -367,10 +383,10 @@ def create_app(backends: List[object], voices: Dict[str, dict], default_voice: O
                                      ref_text: str = Form(""), speaker: str = Form(""), instruct: str = Form(""),
                                      xvec_only: bool = Form(True), temperature: float = Form(0.9), top_k: int = Form(50),
                                      repetition_penalty: float = Form(1.05), voice: str = Form(""), ref_preset: str = Form(""),
-                                     ref_audio: UploadFile = File(None)):
+                                     ref_audio: UploadFile = File(None), seed: Optional[int] = Form(None)):
         """The demo's one-shot endpoint (demo/server.py:546-662): the whole utterance as one base64 WAV plus metrics."""
         req = await demo_request(text, language, mode, ref_text, speaker, instruct, xvec_only, temperature, top_k, repetition_penalty,
-                                 voice, ref_preset, ref_audio)
+                                 voice, ref_preset, ref_audio, seed)
         handle = submit_or_503(req)
         t0 = time.perf_counter()
         parts, sr = [], sample_rate
@@ -412,8 +428,10 @@ def replica_devices(gpus: int, device: str = "cuda") -> List[str]:
     return [f"cuda:{g}" for g in range(gpus)]
 
 
-def build_backends(model: str, gpus: int, max_concurrent: int, chunk_frames: int, max_seq_len: int = 2048, device: str = "cuda"):
-    """One model replica + scheduler per GPU."""
+def build_backends(model: str, gpus: int, max_concurrent: int, chunk_frames: int, max_seq_len: int = 2048, device: str = "cuda",
+                   mixed_policies: bool = False):
+    """One model replica + scheduler per GPU.  mixed_policies: requests of different sampling policies share launches, and a
+    request's `seed` is honoured (serving.BatchScheduler)."""
     import torch
 
     from .model import FasterQwen3TTS
@@ -423,7 +441,7 @@ def build_backends(model: str, gpus: int, max_concurrent: int, chunk_frames: int
     for dev in replica_devices(gpus, device):
         tts = FasterQwen3TTS.from_pretrained(model, device=dev, dtype=torch.bfloat16, max_seq_len=max_seq_len,
                                              max_streams=max_concurrent)
-        out.append(BatchScheduler(tts, chunk_frames=chunk_frames, max_concurrent=max_concurrent).start())
+        out.append(BatchScheduler(tts, chunk_frames=chunk_frames, max_concurrent=max_concurrent, mixed_policies=mixed_policies).start())
     return out
 
 
@@ -461,12 +479,16 @@ def main(argv=None):
     p.add_argument("--max-concurrent", type=int, default=16, help="lock-step streams per GPU")
     p.add_argument("--chunk-frames", type=int, default=8, help="frames per launch = streaming granularity (8 frames = 0.64 s)")
     p.add_argument("--no-warmup", action="store_true", help="open the port at once; the first requests then pay for plan building")
+    p.add_argument("--mixed-policies", action="store_true", dest="mixed_policies",
+                   help="requests of different sampling policies share every launch, and a request's seed is honoured "
+                        "(default: requests are batched with requests of the same policy and a seed is refused)")
     args = p.parse_args(argv)
     logging.basicConfig(level=logging.INFO)
     voices, default_voice = load_voices(args)
     import uvicorn
 
-    backends = build_backends(args.model, args.gpus, args.max_concurrent, args.chunk_frames, device=args.device)
+    backends = build_backends(args.model, args.gpus, args.max_concurrent, args.chunk_frames, device=args.device,
+                              mixed_policies=args.mixed_policies)
     if not args.no_warmup:
         logger.info("Warm-up: %.1f s", warm_up(backends, voices))
     app = create_app(backends, voices, default_voice, sample_rate=backends[0].tts.sample_rate, model_name=args.model)

@@ -14,8 +14,11 @@ requests queue behind each other and a 10-second utterance blocks everyone for 2
 
 A request joins at the next chunk boundary (≤ chunk_frames frame-steps away) and leaves without stopping anyone.  A stream's
 tokens do not depend on its neighbours (batch-invariant arithmetic, DESIGN.md §3.5): under greedy decoding every request's
-codes equal its single-stream run (`tests/test_serving_gpu.py`).  The sampling policy is a launch argument, so requests are
-batched with requests of the same policy; a request with another policy waits for the running cohort to drain.
+codes equal its single-stream run (`tests/test_serving_gpu.py`).  By default the sampling policy is a launch argument, so
+requests are batched with requests of the same policy ("cohorts"); a request with another policy waits for the running cohort
+to drain.  With `mixed_policies=True` every request carries its own policy and seed into its slot (fq3_set_stream_policy):
+requests of any policies share every launch, and a sampled request draws exactly what its single-stream run with the same
+seed draws, whatever slot it got (`tests/test_mixed_policy_gpu.py`).
 
 All engine calls happen on the scheduler's own thread (the engine, like the reference's model, is not thread-safe).
 """
@@ -60,6 +63,7 @@ class TTSRequest:
     top_p: float = 1.0
     do_sample: bool = True
     repetition_penalty: float = 1.05
+    seed: Optional[int] = None  # sampling seed of this request (BatchScheduler(mixed_policies=True)); None: derived from its id
 
     def policy_key(self) -> tuple:
         return (self.do_sample, self.top_k, self.top_p, self.temperature, self.repetition_penalty, self.min_new_tokens)
@@ -139,7 +143,7 @@ class BatchScheduler:
 
     def __init__(self, tts, chunk_frames: int = 8, max_concurrent: Optional[int] = None, seed: int = 0, codec_lanes: int = 4,
                  codec_mode: str = "auto", codec_split_k: Optional[bool] = None, overlap_codec="auto",
-                 emit_every: int = 1):
+                 emit_every: int = 1, mixed_policies: bool = False):
         """codec_mode: "windowed" (default, = "auto") — the reference's 25-frame left-context re-decode (model.py:737-826): the
         audio is bit for bit what the single-stream streaming API returns for the same codes; "stateful" — one
         codec.CodecStream per slot: a chunk costs its own frames and the audio is the full non-streaming decode of the
@@ -158,7 +162,11 @@ class BatchScheduler:
         134–209 audio-s/s run to run.  "auto" (default): "gpu" for up to two utterances in the chunk, "host" beyond.
         "none": codec, host collection, then launch.
         (The first "gpu" runs exposed a missing dependency in the wide frame program — fixed, DESIGN.md §3.5 "pass 0a -> 0b";
-        profiles/r02k_serving_overlap_fault.log, r02k_overlap_stress_after_fix.log.)"""
+        profiles/r02k_serving_overlap_fault.log, r02k_overlap_stress_after_fix.log.)
+        mixed_policies: no cohorts — requests take free slots first come, first served whatever their sampling policy; each
+        admitted request's policy and seed (`TTSRequest.seed`, or one derived from `seed` and the request id) become its slot's
+        own policy before its prefill, and every launch passes one fixed launch-wide policy that no live stream uses.  Off by
+        default: then a request that carries a `seed` is refused (the cohort shares the scheduler's `seed`)."""
         self.tts = tts
         self.emit_every = max(1, int(emit_every))
         self.codec_lanes = max(1, int(codec_lanes))
@@ -180,6 +188,7 @@ class BatchScheduler:
             cap = min(cap, 4)
         self.max_concurrent = min(cap, max_concurrent or cap)
         self.seed = seed
+        self.mixed_policies = bool(mixed_policies)
         self._pending: "queue.Queue[RequestHandle]" = queue.Queue()
         self._deferred: List[RequestHandle] = []   # waiting for the running cohort's policy to drain
         self._active: Dict[int, _Active] = {}
@@ -231,6 +240,11 @@ class BatchScheduler:
             raise ValueError(f"unknown request kind {req.kind!r}")
         if self._failure is not None:  # nobody would ever answer: say so now instead of letting the caller wait for ever
             raise RuntimeError(f"scheduler stopped after a failure: {self._failure!r}")
+        if self.mixed_policies:
+            self._policy(req.policy_key(), 0 if req.seed is None else req.seed).validate()
+        elif req.seed is not None:
+            raise ValueError("a per-request seed needs BatchScheduler(mixed_policies=True): "
+                             "in cohort mode the requests of a launch share the scheduler's seed")
         with self._submit_lock:
             h = RequestHandle(req, self._next_id)
             self._next_id += 1
@@ -257,10 +271,34 @@ class BatchScheduler:
             m, _, _, tie, tam, tth, tpe = t._prepare_generation_custom(r.text, r.language, None, r.instruct)
         return m, tie, tam, tth, tpe, None
 
-    def _policy(self, key: tuple) -> SamplingPolicy:
+    def _policy(self, key: tuple, seed: Optional[int] = None) -> SamplingPolicy:
         do_sample, top_k, top_p, temperature, rep, min_new = key
         return SamplingPolicy(do_sample=do_sample, top_k=top_k, top_p=top_p, temperature=temperature, repetition_penalty=rep,
-                              min_new_tokens=min_new, suppress_tail=1024, seed=self.seed)
+                              min_new_tokens=min_new, suppress_tail=1024, seed=self.seed if seed is None else seed)
+
+    def request_seed(self, h: RequestHandle) -> int:
+        """Mixed mode: the request's own seed, else one derived from the scheduler's seed and the request id (splitmix64), so
+        that it does not depend on the slot the request gets."""
+        if h.request.seed is not None:
+            return int(h.request.seed)
+        x = (int(self.seed) * 0x9E3779B97F4A7C15 + h.id + 1) & 0xFFFFFFFFFFFFFFFF
+        x = ((x ^ (x >> 30)) * 0xBF58476D1CE4E5B9) & 0xFFFFFFFFFFFFFFFF
+        x = ((x ^ (x >> 27)) * 0x94D049BB133111EB) & 0xFFFFFFFFFFFFFFFF
+        return x ^ (x >> 31)
+
+    def _launch_policy(self) -> SamplingPolicy:
+        """The policy argument of a launch: the cohort's, or in mixed mode a fixed one that no live stream uses (every live stream
+        has its own)."""
+        if self.mixed_policies:
+            return SamplingPolicy(do_sample=False, seed=self.seed)
+        return self._policy(self._cohort)
+
+    def _release(self, slot: int):
+        """Retire a slot; in mixed mode also forget its policy, so that a later user of the engine's slot (slot 0: the
+        single-stream API) samples with its own arguments again."""
+        self.eng.retire_stream(slot)
+        if self.mixed_policies:
+            self.eng.set_stream_policy(slot, None)
 
     def _admit(self):
         """Move waiting requests into free slots (prefill runs here, between two chunk launches)."""
@@ -280,7 +318,9 @@ class BatchScheduler:
                 self._finish(h, "cancelled")
                 continue
             key = h.request.policy_key()
-            if self._cohort is None and not self._active:
+            if self.mixed_policies:
+                self._cohort = key  # no cohorts: whatever the policy, the request only waits for a free slot
+            elif self._cohort is None and not self._active:
                 self._cohort = key
             free = [s for s in range(self.max_concurrent) if s not in self._active and s not in self._draining]
             if blocked or key != self._cohort or not free:
@@ -295,10 +335,14 @@ class BatchScheduler:
                         f"Input is too long: prefill has {tie.shape[1]} tokens but max_seq_len={self.eng.max_seq_len}. "
                         "Use shorter text or shorter reference audio.")
                 self.eng.set_text_conditioning(slot, tth[0], tpe)
-                self.eng.prefill(slot, tie[0], _left_pads(tam), self._policy(key))
+                if self.mixed_policies:
+                    self.eng.set_stream_policy(slot, self._policy(key, self.request_seed(h)))
+                    self.eng.prefill(slot, tie[0], _left_pads(tam), self._launch_policy())
+                else:
+                    self.eng.prefill(slot, tie[0], _left_pads(tam), self._policy(key))
             except Exception as e:  # a bad request must not take the loop down
                 try:
-                    self.eng.retire_stream(slot)  # whatever the failed prefill left in the slot must not decode
+                    self._release(slot)  # whatever the failed prefill left in the slot must not decode
                 except Exception:
                     pass
                 h.q.put(e)
@@ -404,7 +448,7 @@ class BatchScheduler:
                 torch.cuda.set_device(eng.device)
             with torch.inference_mode():
                 for s in range(self.eng.max_streams):
-                    eng.retire_stream(s)  # never-used slots idle inside a launch
+                    self._release(s)  # never-used slots idle inside a launch
                 self._backlog = []
                 while not self._stop.is_set():
                     t0 = time.perf_counter()
@@ -434,7 +478,7 @@ class BatchScheduler:
                         self.stats["t_enqueue"] = self.stats.get("t_enqueue", 0.0) + tq - t1
                         self.stats["t_fence"] = self.stats.get("t_fence", 0.0) + time.perf_counter() - tq
                     hi = max(self._active) + 1
-                    eng.decode_frames(hi, self.chunk_frames, self._policy(self._cohort), self.tts.predictor_graph.policy())
+                    eng.decode_frames(hi, self.chunk_frames, self._launch_policy(), self.tts.predictor_graph.policy())
                     t2 = time.perf_counter()
                     self.stats["launches"] += 1
                     self.stats["max_batch"] = max(self.stats["max_batch"], len(self._active))
@@ -474,14 +518,14 @@ class BatchScheduler:
                         elif reason is not None:
                             self._finish(a.handle, reason)
                         if reason is not None:
-                            eng.retire_stream(slot)
+                            self._release(slot)
                             del self._active[slot]
                     self.stats["t_wait"] += time.perf_counter() - t3
                 self._emit(self._backlog)
                 for a in list(self._active.values()):  # stop() in mid-utterance: nobody may wait for ever
                     if a.handle.finish_reason is None:
                         self._finish(a.handle, "shutdown")
-                    eng.retire_stream(a.slot)
+                    self._release(a.slot)
                 self._active.clear()
                 leftover = list(self._deferred)
                 self._deferred = []
