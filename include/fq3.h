@@ -215,6 +215,10 @@ int fq3_set_decode_grid(fq3_engine* e, int n_ctas);
 int fq3_clear_fault(fq3_engine* e, void* stream);
 /* Test hook: set the 32-bit exchange-epoch counter (the wrap-around path is otherwise hours of serving away). */
 int fq3_debug_set_epoch(fq3_engine* e, uint32_t epoch);
+/* Test hook: the first-codebook logits (fp32 [V_t] device, before penalty, suppression and temperature) that stream
+ * `stream_idx`'s last talker sampling phase consumed.  Valid right after an fq3_decode_frames launch of the
+ * reference-shaped program (not the wide one) that ran the stream; -FQ3_E_INVALID otherwise. */
+int fq3_debug_read_talker_logits(fq3_engine* e, int stream_idx, void* out_f32, void* stream);
 /* Copy status / codes back (synchronises `stream`). codes_out: host int32 [n, 16]. */
 int fq3_get_status(fq3_engine* e, int stream_idx, fq3_status* out, void* stream);
 int fq3_read_codes(fq3_engine* e, int stream_idx, int first_frame, int n, int32_t* codes_out, void* stream);

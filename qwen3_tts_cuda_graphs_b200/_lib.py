@@ -80,6 +80,7 @@ SYMBOLS = {
     "fq3_set_decode_grid": (C.c_int, [_P, C.c_int]),
     "fq3_clear_fault": (C.c_int, [_P, _P]),
     "fq3_debug_set_epoch": (C.c_int, [_P, C.c_uint32]),
+    "fq3_debug_read_talker_logits": (C.c_int, [_P, C.c_int, _P, _P]),
     "fq3_get_status": (C.c_int, [_P, C.c_int, C.POINTER(Status), _P]),
     "fq3_read_codes": (C.c_int, [_P, C.c_int, C.c_int, C.c_int, C.POINTER(C.c_int32), _P]),
     "fq3_last_hidden": (C.c_int, [_P, C.c_int, _P, _P]),

@@ -61,6 +61,7 @@ struct fq3_engine {
   int* err_host = nullptr;
   int* err_dev = nullptr;
   float* pred_logits_all = nullptr;
+  int frames_rows = 0;  // streams of the last persistent launch if it ran the reference-shaped frame program, else 0
   uint8_t* seen_scratch = nullptr;
   Phase *d_frames = nullptr, *d_pred = nullptr, *d_talker = nullptr, *d_prefill = nullptr, *d_linear = nullptr, *d_wide = nullptr;
   std::vector<Phase> h_frames, h_pred, h_talker, h_prefill, h_wide;  // host copies (shared-memory sizing)
@@ -442,6 +443,7 @@ int launch(fq3_engine* e, LaunchParams& p, const Phase* prog_host, cudaStream_t 
   void* fn = p.wide ? (void*)fq3_stream_kernel<false, true> : (p.prof ? (void*)fq3_stream_kernel<true, false> : (void*)fq3_stream_kernel<false, false>);
   CK(cudaLaunchCooperativeKernel(fn, dim3(grid), dim3(kThreads), args, smem, s));
   e->launches += 1;
+  e->frames_rows = (p.mode == MODE_FRAMES && !p.wide) ? p.n_rows : 0;
   return 0;
 }
 
@@ -1129,6 +1131,16 @@ int fq3_debug_set_epoch(fq3_engine* e, uint32_t epoch) {
   if (!e || epoch == 0) return fail(FQ3_E_INVALID, "bad arguments");
   e->epoch = epoch;
   return 0;
+}
+
+// The frame program ends with the talker's head and sampler: until the next launch, stream b's BUF_LOGITS row holds the
+// logits its last talker sampling phase consumed (the predictor's heads write that row earlier in the frame).
+int fq3_debug_read_talker_logits(fq3_engine* e, int idx, void* out_f32, void* stream) {
+  if (int r = check_stream(e, idx)) return r;
+  if (!out_f32) return fail(FQ3_E_INVALID, "null output");
+  if (idx >= e->frames_rows)
+    return fail(FQ3_E_INVALID, "the last launch was not a reference-shaped fq3_decode_frames launch that ran this stream");
+  return unpack_f32(e, out_f32, e->tk.d.vocab, BUF_LOGITS, idx, 1, e->tk.d.vocab, (cudaStream_t)stream);
 }
 
 int fq3_get_status(fq3_engine* e, int idx, fq3_status* out, void* stream) {

@@ -2241,7 +2241,7 @@ __device__ __noinline__ int sample_row(const float* logits_g, const LLWord* ll, 
       x = x / a.temperature;
       if (a.round_bf16) x = bf16r(x);
     }
-    sl[i] = x;
+    sl[i] = x + 0.0f;  // -0 -> +0: the top-p step orders by key, and torch's sort puts both zeros in one tie group
   };
   if (ll) {
     // packed words: word w carries logits 2w, 2w+1 (bf16-rounded by the head phase, like the reference's bf16 Linear)
@@ -2294,17 +2294,32 @@ __device__ __noinline__ int sample_row(const float* logits_g, const LLWord* ll, 
     float loc = 0.f;
     for (int i = threadIdx.x; i < V; i += kConsumerThreads) loc += expf(sl[i] - vmax);
     const float total = block_sum(loc, sc.redf);
-    const float P = a.top_p * total;
-    uint32_t lo = 0u, hi = 0xffffffffu;  // smallest key t with mass(key >= t) <= P
+    // fp32: unnormalised masses against top_p * total.  bf16 (the reference's softmax and cumsum of a bf16 tensor, compared
+    // with bf16(top_p)): every probability rounded to bf16, and the prefix kept while it would round to at most bf16(top_p),
+    // i.e. up to the midpoint P between bf16(top_p) and the next bf16 value.  A prefix exactly on P rounds to the even one of
+    // the two, so it is kept iff bf16(top_p) is even (`strict` otherwise).  Both masses grow with the key.
+    const bool bf = a.round_bf16;
+    auto mass = [&](float x) {
+      const float e = expf(x - vmax);
+      return bf ? bf16r(e / total) : e;
+    };
+    float P = a.top_p * total;
+    bool strict = false;
+    if (bf) {
+      const uint32_t b = __float_as_uint(bf16r(a.top_p));
+      P = 0.5f * (__uint_as_float(b) + __uint_as_float(b + 0x10000u));
+      strict = (b & 0x10000u) != 0;
+    }
+    uint32_t lo = 0u, hi = 0xffffffffu;  // smallest key t with mass(key >= t) <= P (< P when strict)
     for (int it = 0; it < 32; ++it) {
       const uint32_t mid = lo + ((hi - lo) >> 1);
       float msum = 0.f;
       for (int i = threadIdx.x; i < V; i += kConsumerThreads) {
         const float x = sl[i];
-        if (f2key(x) >= mid) msum += expf(x - vmax);
+        if (f2key(x) >= mid) msum += mass(x);
       }
       msum = block_sum(msum, sc.redf);
-      if (msum <= P) hi = mid; else lo = mid + 1;
+      if (msum < P || (!strict && msum == P)) hi = mid; else lo = mid + 1;
     }
     const uint32_t tkey = hi;
     // boundary value v* = largest key below tkey; its first j ties (index order) may still fit under P
@@ -2316,12 +2331,13 @@ __device__ __noinline__ int sample_row(const float* logits_g, const LLWord* ll, 
     const float bval = block_max(key2f(bk), sc.redf);
     float above = 0.f;
     for (int i = threadIdx.x; i < V; i += kConsumerThreads)
-      if (f2key(sl[i]) >= tkey) above += expf(sl[i] - vmax);
+      if (f2key(sl[i]) >= tkey) above += mass(sl[i]);
     above = block_sum(above, sc.redf);
     int keep_ties = 0;
     if (bval > -INFINITY) {
-      const float pe = expf(bval - vmax);
+      const float pe = mass(bval);
       keep_ties = (int)floorf((P - above) / pe);
+      if (strict && above + (float)keep_ties * pe >= P) --keep_ties;  // bf16 masses: these sums are exact
       if (keep_ties < 0) keep_ties = 0;
     }
     const int seg = (V + kConsumerThreads - 1) / kConsumerThreads;

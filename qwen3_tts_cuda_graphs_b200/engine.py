@@ -284,6 +284,12 @@ class Engine:
         pol, s = policy.c(), sub.c()
         _lib.check(self.lib.fq3_decode_frames(self.h, int(n_streams), int(n_frames), C.byref(pol), C.byref(s), _stream()))
 
+    def debug_talker_logits(self, idx: int = 0) -> torch.Tensor:
+        """fp32 [V_t]: the logits stream idx's last talker sampler consumed, right after decode_frames (fq3.h test hook)."""
+        out = torch.empty(self.cfg.talker.vocab_size, dtype=torch.float32, device=self.device)
+        _lib.check(self.lib.fq3_debug_read_talker_logits(self.h, int(idx), out.data_ptr(), _stream()))
+        return out
+
     def last_hidden(self, row: int = 0) -> torch.Tensor:
         out = torch.empty(self.cfg.talker.hidden_size, dtype=torch.bfloat16, device=self.device)
         _lib.check(self.lib.fq3_last_hidden(self.h, int(row), out.data_ptr(), _stream()))

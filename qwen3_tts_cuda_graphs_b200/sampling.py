@@ -2,8 +2,8 @@
 
 Same call signatures as the reference's `faster_qwen3_tts/sampling.py:10-66`; the arithmetic runs in one
 block-wide kernel of libfq3.so (`fq3_sample`, csrc/fq3_kernel.cuh `sample_row`) instead of ~15 ATen launches
-with two host synchronisations (SURVEY.md §2c).  The draw uses a counter-based Philox stream, so sampling
-parity with torch.multinomial is statistical, while greedy / top-k sets / penalties are exact.
+with two host synchronisations (SURVEY.md §2c).  The draw uses a counter-based Philox stream, so the draws are not
+torch.multinomial's, while greedy / top-k and top-p sets / penalties are exact; oracle/sampler_oracle.py replays every draw.
 """
 from __future__ import annotations
 
