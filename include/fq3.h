@@ -80,7 +80,8 @@ typedef struct fq3_subpolicy {
 /* Host-visible per-stream status after fq3_decode_frames (streaming.py:157-188 needs steps + is_final). */
 typedef struct fq3_status {
   int32_t n_frames;  /* frames appended so far for this utterance */
-  int32_t done;      /* 0 running, 1 EOS sampled (generate.py:150), 2 static cache full (generate.py:175-177), 3 retired by the host */
+  int32_t done;      /* 0 running, 1 EOS sampled (generate.py:150), 2 static cache full (generate.py:175-177), 3 retired by the host,
+                        4 waiting for text (fq3_open_text): not finished, resumes after fq3_append_text */
   int32_t position;  /* next KV position */
   int32_t gen_step;  /* generate.py:199 */
   int32_t token;     /* first-codebook id that will open the next frame */
@@ -127,9 +128,25 @@ int fq3_retire_stream(fq3_engine* e, int stream_idx, void* stream);
 /* TalkerGraph.set_generation_state (talker_graph.py:172-196): left pads and rope delta of one stream. */
 int fq3_set_generation_state(fq3_engine* e, int stream_idx, int n_left_pad, int rope_delta, void* stream);
 /* trailing_text_hiddens / tts_pad_embed of generate.py:168-171; copied into engine-owned buffers.
- * trailing: bf16 [n_trailing, H_t]; pad_embed: bf16 [H_t]. */
+ * trailing: bf16 [n_trailing, H_t]; pad_embed: bf16 [H_t].  The text is closed: it ends after these rows, also on a slot
+ * whose text was open (fq3_open_text). */
 int fq3_set_text_conditioning(fq3_engine* e, int stream_idx, const void* trailing, int n_trailing,
                               const void* pad_embed, void* stream);
+/* Incremental text input (no counterpart in the reference): the trailing text rows of a stream arrive while it decodes.
+ * fq3_open_text empties the stream's trailing text and leaves it open; fq3_append_text copies rows bf16 [n, H_t] after the
+ * rows given so far and, with close != 0, ends the text (later frames add pad_embed, as after the last row of a closed text).
+ * A frame of an open stream that needs text row gen_step before it has arrived is not run: the stream's sampler sets
+ * status.done = 4 ("waiting for text") and the stream idles, its state unchanged, through the rest of the launch and every
+ * later launch until an fq3_append_text delivers that row or closes the text, which sets done back to 0.  A wait changes no
+ * arithmetic and no draw: whatever the arrival schedule, the stream's codes are the codes of the same stream with the whole
+ * text given up front by fq3_set_text_conditioning.  A prefill of an open stream whose text has no row yet ends waiting.
+ * A launch whose streams all wait runs one idle frame: the caller skips it.  Both calls are stream-ordered (a kernel on
+ * `stream` updates the state; the rows may be freed once `stream` has passed the call) and must not overlap a launch on the
+ * stream.  The open state survives fq3_reset_stream and the reset inside a prefill, as the text rows do;
+ * fq3_set_text_conditioning closes it.  fq3_append_text returns -FQ3_E_INVALID when the stream's text is not open and
+ * -FQ3_E_TOO_LONG when the rows would exceed max_seq_len. */
+int fq3_open_text(fq3_engine* e, int stream_idx, const void* pad_embed, void* stream);
+int fq3_append_text(fq3_engine* e, int stream_idx, const void* rows, int n, int close, void* stream);
 /* TalkerGraph.prefill_kv (talker_graph.py:153-170): import an externally computed prefix KV.
  * k, v: bf16 [n_kv_heads, T, head_dim] of one layer.  Returns -FQ3_E_TOO_LONG if T > max_seq_len
  * (the reference raises RuntimeError, talker_graph.py:163-167). */

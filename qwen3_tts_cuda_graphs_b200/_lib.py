@@ -63,6 +63,8 @@ SYMBOLS = {
     "fq3_set_stream_policy": (C.c_int, [_P, C.c_int, C.POINTER(Policy), _P]),
     "fq3_set_generation_state": (C.c_int, [_P, C.c_int, C.c_int, C.c_int, _P]),
     "fq3_set_text_conditioning": (C.c_int, [_P, C.c_int, _P, C.c_int, _P, _P]),
+    "fq3_open_text": (C.c_int, [_P, C.c_int, _P, _P]),
+    "fq3_append_text": (C.c_int, [_P, C.c_int, _P, C.c_int, C.c_int, _P]),
     "fq3_import_kv": (C.c_int, [_P, C.c_int, C.c_int, _P, _P, C.c_int, _P]),
     "fq3_set_loop_state": (C.c_int, [_P, C.c_int, C.c_int, _P, C.c_int, C.c_int, _P]),
     "fq3_prefill": (C.c_int, [_P, C.c_int, _P, C.c_int, C.c_int, C.POINTER(Policy), _P, _P]),

@@ -56,6 +56,8 @@ struct fq3_engine {
   std::vector<uint8_t> spol_on;    // host mirror of the records' `on` flags, in call order: a launch none of whose streams has a
                                    // record gets no record pointer, so its samplers issue no extra load on the critical path
   std::vector<StreamState> h_st;
+  std::vector<int> text_rows;      // per stream: text rows given by the host (n_trailing; only host calls change it)
+  std::vector<uint8_t> text_open;  // per stream: fq3_open_text was called and the text has not been closed since
   LLWord* attn_part = nullptr;
   size_t attn_part_bytes = 0;
   int* err_host = nullptr;
@@ -641,6 +643,8 @@ static int create_impl(const fq3_model_desc* desc, fq3_engine* e) {
   e->h_st.resize(B);
   e->in_wpin.assign(B, 0);
   e->spol_on.assign(B, 0);
+  e->text_rows.assign(B, 0);
+  e->text_open.assign(B, 0);
   if (dalloc(e, &e->d_st, B)) return -FQ3_E_CUDA;
   if (dalloc(e, &e->d_spol, B)) return -FQ3_E_CUDA;
   for (int b = 0; b < B; ++b) {
@@ -649,6 +653,7 @@ static int create_impl(const fq3_model_desc* desc, fq3_engine* e) {
     bf16 *tr = nullptr, *pe = nullptr;
     if (dalloc(e, &tr, (size_t)e->tk.d.max_pos * Ht)) return -FQ3_E_CUDA;
     if (dalloc(e, &pe, (size_t)Ht)) return -FQ3_E_CUDA;
+    if (dalloc(e, &s.held, (size_t)Ht)) return -FQ3_E_CUDA;
     if (dalloc(e, &s.codes, (size_t)desc->max_frames * desc->n_code_groups)) return -FQ3_E_CUDA;
     if (dalloc(e, &s.seen, (size_t)round_up(e->tk.d.vocab, 16))) return -FQ3_E_CUDA;
     s.trailing = tr;
@@ -795,7 +800,41 @@ int fq3_set_text_conditioning(fq3_engine* e, int idx, const void* trailing, int 
     CK(cudaMemcpyAsync(const_cast<bf16*>(e->h_st[idx].trailing), trailing, (size_t)n_trailing * Ht * 2,
                        cudaMemcpyDeviceToDevice, s));
   CK(cudaMemcpyAsync(const_cast<bf16*>(e->h_st[idx].pad_embed), pad_embed, (size_t)Ht * 2, cudaMemcpyDeviceToDevice, s));
-  fq3_set_state_kernel<<<1, 32, 0, s>>>(e->d_st + idx, 0, 0, 0, 4, 0, 0, n_trailing);
+  fq3_set_state_kernel<<<1, 32, 0, s>>>(e->d_st + idx, 0, 0, 0, 4, 0, 0, n_trailing);  // closed text
+  e->text_rows[idx] = n_trailing;
+  e->text_open[idx] = 0;
+  e->launches += 1;
+  CK(cudaGetLastError());
+  return 0;
+}
+
+int fq3_open_text(fq3_engine* e, int idx, const void* pad_embed, void* stream) {
+  if (int r = check_stream(e, idx)) return r;
+  if (!pad_embed) return fail(FQ3_E_INVALID, "null pad_embed");
+  cudaStream_t s = (cudaStream_t)stream;
+  CK(cudaMemcpyAsync(const_cast<bf16*>(e->h_st[idx].pad_embed), pad_embed, (size_t)e->tk.d.hidden * 2, cudaMemcpyDeviceToDevice, s));
+  fq3_set_state_kernel<<<1, 32, 0, s>>>(e->d_st + idx, 0, 0, 0, 4 | 64, 0, 0, 0);
+  e->text_rows[idx] = 0;
+  e->text_open[idx] = 1;
+  e->launches += 1;
+  CK(cudaGetLastError());
+  return 0;
+}
+
+int fq3_append_text(fq3_engine* e, int idx, const void* rows, int n, int close, void* stream) {
+  if (int r = check_stream(e, idx)) return r;
+  if (!e->text_open[idx]) return fail(FQ3_E_INVALID, "the stream's text is not open (fq3_open_text)");
+  if (n < 0 || (n > 0 && !rows)) return fail(FQ3_E_INVALID, "bad text rows");
+  const int total = e->text_rows[idx] + n;
+  if (total > e->tk.d.max_pos) return fail(FQ3_E_TOO_LONG, "trailing text longer than max_seq_len");
+  cudaStream_t s = (cudaStream_t)stream;
+  const int Ht = e->tk.d.hidden;
+  if (n > 0)
+    CK(cudaMemcpyAsync(const_cast<bf16*>(e->h_st[idx].trailing) + (size_t)e->text_rows[idx] * Ht, rows, (size_t)n * Ht * 2,
+                       cudaMemcpyDeviceToDevice, s));
+  fq3_set_state_kernel<<<1, 32, 0, s>>>(e->d_st + idx, 0, 0, 0, close ? 4 : 4 | 64, 0, 0, total);
+  e->text_rows[idx] = total;
+  e->text_open[idx] = close ? 0 : 1;
   e->launches += 1;
   CK(cudaGetLastError());
   return 0;

@@ -176,9 +176,11 @@ struct StreamState {  // one per stream, device memory
   int n_pad;
   int rope_delta;
   int n_trailing;
+  int text_open;          // fq3_open_text: rows past n_trailing may still arrive; a frame that needs one waits (done = 4)
   unsigned long long draws;
   const bf16* trailing;   // [n_trailing, H_t]
   const bf16* pad_embed;  // [H_t]
+  bf16* held;             // [H_t] past_hidden of a waiting stream (done = 4): its BUF_HID row is overwritten while it idles
   int* codes;             // [max_frames, 16]
   uint8_t* seen;          // [V_t] first-codebook history bitmap (repetition penalty)
   int cur_codes[32];

@@ -2636,6 +2636,15 @@ __device__ __forceinline__ int sample_ll(const LLWord* ll, uint32_t ep, const La
 __device__ __forceinline__ void publish_row(LLWord* dst, const bf16* src, int n, uint32_t ep) {
   for (int c = threadIdx.x; c < (n >> 1); c += kConsumerThreads) ll_st(dst + c, __ldg(reinterpret_cast<const uint32_t*>(src) + c), ep);
 }
+// The same for a waiting stream's held row, which this kernel wrote: read through L2, not the read-only path.
+__device__ __noinline__ void publish_held_row(LLWord* dst, const bf16* src, int n, uint32_t ep) {
+  for (int c = threadIdx.x; c < (n >> 1); c += kConsumerThreads) ll_st(dst + c, __ldcg(reinterpret_cast<const uint32_t*>(src) + c), ep);
+}
+// Keep a stream's past_hidden row when it starts waiting for text: each thread copies the words it publishes from held later.
+__device__ __noinline__ void hold_row(bf16* dst, const bf16* src, int n) {
+  for (int c = threadIdx.x; c < (n >> 1); c += kConsumerThreads)
+    __stcg(reinterpret_cast<uint32_t*>(dst) + c, __ldg(reinterpret_cast<const uint32_t*>(src) + c));
+}
 
 template <bool WIDE>
 __device__ __forceinline__ void sample_phase(const Phase& ph, const LaunchParams& p, unsigned char* smem_base, uint32_t ep, int pidx,
@@ -2757,6 +2766,8 @@ __device__ __forceinline__ void sample_phase(const Phase& ph, const LaunchParams
       if (live) {
         if (ph.skind == SMP_TALKER) { new_pos += 1; new_gs += 1; }
         if (tok == p.eos_id) new_done = 1;  // generate.py:150 — checked before the next frame is built
+        // open text (fq3_open_text): the next frame adds text row new_gs; until it has arrived the stream waits, state unchanged
+        else if (__ldcg(&st->text_open) && new_gs >= __ldcg(&st->n_trailing)) new_done = 4;
       } else {
         tok = __ldcg(&st->token);
       }
@@ -2768,14 +2779,21 @@ __device__ __forceinline__ void sample_phase(const Phase& ph, const LaunchParams
         ll_st(&st->ctl[1], (uint32_t)new_pos, ep);
       }
       // predictor pass-0 input rows [past_hidden ; codec_embed(token)] (generate.py:154-155), addressed by
-      // stream slot; always re-published so every reader sees this phase's epoch
+      // stream slot; always re-published so every reader sees this phase's epoch.  A waiting stream's BUF_HID row is the
+      // result of an idle talker pass: its past_hidden comes from the row it held when it started waiting.
       const bf16* hid = reinterpret_cast<const bf16*>(p.bufs[BUF_HID]) + (size_t)b * p.ld[BUF_HID];
-      if constexpr (WIDE) {  // the wide program keeps them in BUF_WPIN (the host converts between the two layouts: fq3_api.cu, sync_pin_layout)
-        LLWord* wp = reinterpret_cast<LLWord*>(p.bufs[BUF_WPIN]);
-        publish_row(wp + (size_t)slot * p.ld[BUF_WPIN], hid, Ht, ep);
-        publish_row(wp + (size_t)(p.max_streams + slot) * p.ld[BUF_WPIN], p.codec_embed + (size_t)tok * Ht, Ht, ep);
+      LLWord* const hid_dst = WIDE ? reinterpret_cast<LLWord*>(p.bufs[BUF_WPIN]) + (size_t)slot * p.ld[BUF_WPIN]
+                                   : pin + (size_t)(2 * slot) * ldpin;
+      if (done_now == 4) {
+        publish_held_row(hid_dst, st->held, Ht, ep);
       } else {
-        publish_row(pin + (size_t)(2 * slot) * ldpin, hid, Ht, ep);
+        if (new_done == 4) hold_row(st->held, hid, Ht);
+        publish_row(hid_dst, hid, Ht, ep);
+      }
+      if constexpr (WIDE) {  // the wide program keeps them in BUF_WPIN (the host converts between the two layouts: fq3_api.cu, sync_pin_layout)
+        publish_row(reinterpret_cast<LLWord*>(p.bufs[BUF_WPIN]) + (size_t)(p.max_streams + slot) * p.ld[BUF_WPIN],
+                    p.codec_embed + (size_t)tok * Ht, Ht, ep);
+      } else {
         publish_row(pin + (size_t)(2 * slot + 1) * ldpin, p.codec_embed + (size_t)tok * Ht, Ht, ep);
       }
       if (threadIdx.x == 0) __threadfence();  // once per step: K/V rows stored by this CTA (see above)
@@ -3086,7 +3104,12 @@ __global__ void fq3_set_state_kernel(StreamState* st, int token, int position, i
   if (threadIdx.x == 0) {
     if (set_mask & 1) st->token = token;
     if (set_mask & 2) { st->n_pad = n_pad; st->rope_delta = rope_delta; }
-    if (set_mask & 4) st->n_trailing = n_trailing;
+    if (set_mask & 4) {  // text conditioning: n_trailing rows, still open (64) or closed
+      st->n_trailing = n_trailing;
+      st->text_open = (set_mask & 64) ? 1 : 0;
+      // a stream waiting for text runs again once its next row has arrived or its text has ended
+      if (st->done == 4 && (!(set_mask & 64) || st->gen_step < n_trailing)) st->done = 0;
+    }
     if (set_mask & 8) { st->position = position; st->gen_step = gen_step; }
     if (set_mask & 16) st->done = 0;
     if (set_mask & 32) st->done = 3;  // retired by the host (fq3_retire_stream): idles in lock-step launches until reset

@@ -183,6 +183,21 @@ class Engine:
         _lib.check(self.lib.fq3_set_text_conditioning(self.h, idx, tr.data_ptr(), tr.shape[0], pe.data_ptr(), _stream()))
         self._cond_ref = (tr, pe)
 
+    def open_text(self, idx: int, pad_embed: torch.Tensor):
+        """Empty the stream's trailing text and leave it open: its rows arrive through append_text while it decodes, and a frame
+        whose text row has not arrived waits (status.done = 4) instead of running (fq3.h: fq3_open_text)."""
+        pe = self._bf16(pad_embed.reshape(self.cfg.talker.hidden_size))
+        _lib.check(self.lib.fq3_open_text(self.h, int(idx), pe.data_ptr(), _stream()))
+        self._open_ref = pe
+
+    def append_text(self, idx: int, rows: torch.Tensor, close: bool = False):
+        """Append bf16 text rows [n, H_t] to an open stream's trailing text; close=True ends the text (fq3.h: fq3_append_text).
+        Fq3Error when the stream's text is not open, RuntimeError past max_seq_len rows."""
+        r = self._bf16(rows.reshape(-1, self.cfg.talker.hidden_size))
+        ptr = r.data_ptr() if r.shape[0] > 0 else None
+        _lib.check(self.lib.fq3_append_text(self.h, int(idx), ptr, int(r.shape[0]), int(bool(close)), _stream()))
+        self._append_ref = r
+
     def import_kv(self, idx: int, layer: int, k: torch.Tensor, v: torch.Tensor):
         k, v = self._bf16(k), self._bf16(v)  # [nkv, T, d]
         self._kv_ref = (k, v)

@@ -13,7 +13,7 @@ import logging
 import os
 import wave
 from pathlib import Path
-from typing import Generator, List, Optional, Tuple, Union
+from typing import Generator, Iterable, List, Optional, Tuple, Union
 
 import numpy as np
 import torch
@@ -482,6 +482,33 @@ class FasterQwen3TTS:
                     top_p=top_p, do_sample=do_sample, repetition_penalty=repetition_penalty,
                     predictor_graph=self.predictor_graph, talker_graph=self.talker_graph)
 
+    # ---- streaming text ------------------------------------------------------------------------
+    def _prepare_custom_open(self, text, language, speaker, instruct):
+        _, talker, _, tie, tam, _, tpe = self._prepare_generation_custom(text, language, speaker, instruct)
+        return tie, tam, tpe, talker
+
+    def _generate_open_text(self, pieces, prepare, chunk_size, max_new_tokens, min_new_tokens, temperature, top_k, top_p,
+                            do_sample, repetition_penalty):
+        """The `*_streaming` generators with `text` an iterable of str pieces (an LLM's token stream, say): speech starts after
+        the first committed text token and the stream waits on the device whenever its next text token has not arrived
+        (text_stream.py).  Codes and audio equal the `str` call's on the whole text (text_stream.py: up to ~120 text tokens)."""
+        from .generate import _fresh_seed, is_fused
+        from .text_stream import TextFeed, generate_open
+
+        m = self.model.model
+        if not is_fused(m.talker, self.predictor_graph, self.talker_graph):
+            raise ValueError("streaming text runs on the fused engine path only, not on the operator-at-a-time path")
+        feed = TextFeed(self.model.tokenizer.assistant, m.config.tts_eos_token_id)
+
+        def make_policy():
+            return SamplingPolicy(do_sample=do_sample, top_k=top_k, top_p=top_p, temperature=temperature,
+                                  repetition_penalty=repetition_penalty, min_new_tokens=min_new_tokens, suppress_tail=1024,
+                                  seed=_fresh_seed())
+
+        stream = generate_open(self.talker_graph, self.predictor_graph, prepare, feed, pieces, make_policy, max_new_tokens,
+                               chunk_size)
+        yield from self._stream_audio(m, stream, None, chunk_size)
+
     # ---- voice clone ---------------------------------------------------------------------------
     @torch.inference_mode()
     def generate_voice_clone(self, text: str, language: str, ref_audio, ref_text: str, max_new_tokens: int = 2048,
@@ -553,7 +580,7 @@ class FasterQwen3TTS:
         return audio, self.sample_rate
 
     @torch.inference_mode()
-    def generate_voice_clone_streaming(self, text: str, language: str, ref_audio, ref_text: str,
+    def generate_voice_clone_streaming(self, text: Union[str, Iterable[str]], language: str, ref_audio, ref_text: str,
                                        max_new_tokens: int = 2048, min_new_tokens: int = 2, temperature: float = 0.9,
                                        top_k: int = 50, top_p: float = 1.0, do_sample: bool = True,
                                        repetition_penalty: float = 1.05, chunk_size: int = 12, xvec_only: bool = True,
@@ -563,6 +590,21 @@ class FasterQwen3TTS:
 
         if parity_mode:
             raise NotImplementedError("parity_mode runs upstream qwen_tts with a dynamic cache (streaming.py:192-359); not part of this engine")
+        if not isinstance(text, str):
+            if not xvec_only:
+                raise ValueError("streaming text: an ICL voice clone sums the text into the reference-code rows; use xvec_only=True")
+            if non_streaming_mode:
+                raise ValueError("streaming text needs non_streaming_mode=False (the whole text is in the prompt otherwise)")
+
+            def prepare(s):
+                m, talker, _, tie, tam, _, tpe, _ = self._prepare_generation(
+                    s, ref_audio, ref_text, language=language, xvec_only=True, non_streaming_mode=False,
+                    append_silence=append_silence, instruct=instruct)
+                return tie, tam, tpe, talker
+
+            yield from self._generate_open_text(text, prepare, chunk_size, max_new_tokens, min_new_tokens, temperature, top_k, top_p,
+                                                do_sample, repetition_penalty)
+            return
         m, talker, config, tie, tam, tth, tpe, ref_codes = self._prepare_generation(
             text, ref_audio, ref_text, language=language, xvec_only=xvec_only, non_streaming_mode=non_streaming_mode,
             append_silence=append_silence, instruct=instruct)
@@ -600,7 +642,7 @@ class FasterQwen3TTS:
         return audio, sr
 
     @torch.inference_mode()
-    def generate_custom_voice_streaming(self, text: str, speaker: str, language: str, instruct: Optional[str] = None,
+    def generate_custom_voice_streaming(self, text: Union[str, Iterable[str]], speaker: str, language: str, instruct: Optional[str] = None,
                                         max_new_tokens: int = 2048, min_new_tokens: int = 2, temperature: float = 0.9,
                                         top_k: int = 50, top_p: float = 1.0, do_sample: bool = True,
                                         repetition_penalty: float = 1.05, chunk_size: int = 12):
@@ -609,6 +651,11 @@ class FasterQwen3TTS:
         self._check_custom(language, speaker)
         if self.model.model.tts_model_size in "0b6":
             instruct = None
+        if not isinstance(text, str):
+            yield from self._generate_open_text(
+                text, lambda s: self._prepare_custom_open(s, language, speaker, instruct), chunk_size, max_new_tokens,
+                min_new_tokens, temperature, top_k, top_p, do_sample, repetition_penalty)
+            return
         m, talker, config, tie, tam, tth, tpe = self._prepare_generation_custom(text, language, speaker, instruct)
         stream = fast_generate_streaming(
             talker=talker, talker_input_embeds=tie, attention_mask=tam, trailing_text_hiddens=tth, tts_pad_embed=tpe,
@@ -641,13 +688,18 @@ class FasterQwen3TTS:
         return audio, sr
 
     @torch.inference_mode()
-    def generate_voice_design_streaming(self, text: str, instruct: str, language: str, max_new_tokens: int = 2048,
+    def generate_voice_design_streaming(self, text: Union[str, Iterable[str]], instruct: str, language: str, max_new_tokens: int = 2048,
                                         min_new_tokens: int = 2, temperature: float = 0.9, top_k: int = 50,
                                         top_p: float = 1.0, do_sample: bool = True, repetition_penalty: float = 1.05,
                                         chunk_size: int = 12):
         from .streaming import fast_generate_streaming
 
         self._check_design(language)
+        if not isinstance(text, str):
+            yield from self._generate_open_text(
+                text, lambda s: self._prepare_custom_open(s, language, None, instruct), chunk_size, max_new_tokens,
+                min_new_tokens, temperature, top_k, top_p, do_sample, repetition_penalty)
+            return
         m, talker, config, tie, tam, tth, tpe = self._prepare_generation_custom(text, language, None, instruct)
         stream = fast_generate_streaming(
             talker=talker, talker_input_embeds=tie, attention_mask=tam, trailing_text_hiddens=tth, tts_pad_embed=tpe,

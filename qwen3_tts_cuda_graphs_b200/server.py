@@ -10,6 +10,10 @@ concurrent requests decode in lock-step on the same weight sweep, one scheduler 
     python -m qwen3_tts_cuda_graphs_b200.server --model <dir | synthetic://0.6B-Base> --ref-audio voice.wav --ref-text "..." \
         [--voices voices.json] [--gpus 8] [--max-concurrent 16] [--port 8000]
 
+Text that is still arriving (an LLM's reply) goes through the WebSocket `/v1/audio/speech/stream`: a JSON `{voice, seed?,
+response_format: "pcm"}`, then `{"text": ...}` messages and `{"close": true}`; PCM16 chunks come back as they are decoded, then
+`{"event": "done", "finish_reason", "frames"}`.
+
 `create_app(backends, voices, default_voice)` takes anything with the scheduler's `submit(TTSRequest) -> handle` surface, so the
 HTTP layer is tested on CPU with a stand-in backend (`tests/test_server_cpu.py`).
 """
@@ -31,7 +35,7 @@ import time
 from typing import Dict, List, Optional
 
 import numpy as np
-from fastapi import FastAPI, File, Form, HTTPException, UploadFile  # module level: the endpoints' annotations are resolved by name
+from fastapi import FastAPI, File, Form, HTTPException, UploadFile, WebSocket, WebSocketDisconnect  # module level: the endpoints' annotations are resolved by name
 from fastapi.responses import JSONResponse, Response, StreamingResponse
 from pydantic import BaseModel
 from starlette.background import BackgroundTask
@@ -377,6 +381,78 @@ def create_app(backends: List[object], voices: Dict[str, dict], default_voice: O
 
         return StreamingResponse(sse(), media_type="text/event-stream", headers={"Cache-Control": "no-cache", "X-Accel-Buffering": "no"},
                                  background=BackgroundTask(settle, handle))
+
+    @app.websocket("/v1/audio/speech/stream")
+    async def speech_stream(ws: WebSocket):
+        """Text that is still arriving (an LLM's reply) in, PCM16 out.  First message: JSON {"voice", "seed"?, "response_format":
+        "pcm"}; then any number of {"text": "..."} and one {"close": true}.  The server answers with binary PCM16 chunks as they
+        are decoded and a final {"event": "done", "finish_reason", "frames"}; bad input gets {"event": "error", "detail"} and close
+        code 1008.  MAX_TEXT_CHARS bounds the whole text.  A disconnect cancels the request (serving.TTSRequest(text_open=True))."""
+        await ws.accept()
+        handle, sender = None, None
+
+        async def refuse(detail: str, code: int = 1008):
+            await ws.send_json({"event": "error", "detail": detail})
+            await ws.close(code=code)
+
+        try:
+            first = await ws.receive_json()
+            if not isinstance(first, dict) or "voice" not in first:
+                return await refuse('the first message must be a JSON object {"voice": ..., "response_format": "pcm"}')
+            if str(first.get("response_format", "pcm")).lower() != "pcm":
+                return await refuse("response_format must be 'pcm' on this endpoint")
+            try:
+                voice_cfg = resolve_voice(str(first["voice"]))
+                handle = disp.submit(_request_for(voice_cfg, "", {"seed": first.get("seed"), "text_open": True}))
+            except HTTPException as e:
+                return await refuse(str(e.detail))
+            except ValueError as e:
+                return await refuse(str(e))
+            except RuntimeError as e:  # no healthy backend
+                return await refuse(str(e), 1011)
+
+            async def pump():
+                frames = 0
+                try:
+                    async for audio, _sr, info in chunks_of(handle):
+                        frames += int(info.get("chunk_steps", 0))
+                        await ws.send_bytes(to_pcm16(audio))
+                except ValueError as e:  # e.g. the text closed empty
+                    return await refuse(str(e))
+                except Exception as e:
+                    return await refuse(str(e), 1011)
+                await ws.send_json({"event": "done", "finish_reason": handle.finish_reason, "frames": frames})
+                await ws.close()
+
+            sender = asyncio.ensure_future(pump())
+            total = 0
+            while True:
+                recv = asyncio.ensure_future(ws.receive_json())
+                done, _ = await asyncio.wait({recv, sender}, return_when=asyncio.FIRST_COMPLETED)
+                if recv not in done:  # the request ended first (length cap, error): nothing more to read
+                    recv.cancel()
+                    return
+                msg = recv.result()
+                if isinstance(msg, dict) and "text" in msg and isinstance(msg["text"], str):
+                    total += len(msg["text"])
+                    if total > MAX_TEXT_CHARS:
+                        return await refuse(f"Text too long ({total} chars). Maximum is {MAX_TEXT_CHARS} characters.")
+                    handle.push_text(msg["text"])
+                elif isinstance(msg, dict) and msg.get("close") is True:
+                    handle.close_text()
+                    break
+                else:
+                    return await refuse('expected {"text": "..."} or {"close": true}')
+            await sender
+        except WebSocketDisconnect:
+            pass
+        except ValueError:  # not JSON
+            await refuse("messages must be JSON")
+        finally:  # a disconnect or a refusal cancels what is still decoding
+            if sender is not None and not sender.done():
+                sender.cancel()
+            if handle is not None:
+                settle(handle)
 
     @app.post("/generate")
     async def generate_non_streaming(text: str = Form(...), language: str = Form("English"), mode: str = Form("voice_clone"),

@@ -20,6 +20,12 @@ to drain.  With `mixed_policies=True` every request carries its own policy and s
 requests of any policies share every launch, and a sampled request draws exactly what its single-stream run with the same
 seed draws, whatever slot it got (`tests/test_mixed_policy_gpu.py`).
 
+A request can also be open (`TTSRequest(text_open=True)`): its text keeps arriving through `RequestHandle.push_text` /
+`close_text`.  It is admitted once its first text token is committed (text_stream.TextFeed), the pieces it received are appended
+to its slot before every launch, a stream waiting for text (status.done = 4) counts as running, no launch happens while every
+running stream waits, and its audio goes out in whole chunks of `chunk_frames`, so it equals the one-shot run's.  A request whose
+text stays silent for `text_timeout` seconds is cancelled.
+
 All engine calls happen on the scheduler's own thread (the engine, like the reference's model, is not thread-safe).
 """
 from __future__ import annotations
@@ -64,6 +70,7 @@ class TTSRequest:
     do_sample: bool = True
     repetition_penalty: float = 1.05
     seed: Optional[int] = None  # sampling seed of this request (BatchScheduler(mixed_policies=True)); None: derived from its id
+    text_open: bool = False  # the text keeps arriving: `text` is its first piece, RequestHandle.push_text / close_text the rest
 
     def policy_key(self) -> tuple:
         return (self.do_sample, self.top_k, self.top_p, self.temperature, self.repetition_penalty, self.min_new_tokens)
@@ -83,9 +90,45 @@ class RequestHandle:
         self.finish_reason: Optional[str] = None
         self.cancelled = False
         self._sr = 24000
+        self._wake: Optional[threading.Event] = None  # the scheduler's: set when text arrives or the request is cancelled
+        self._text_lock = threading.Lock()
+        self._pieces: List[str] = [req.text] if req.text_open and req.text else []
+        self._text_closed = not req.text_open
+        self._t_text = time.monotonic()  # when text last arrived (TTSRequest(text_open=True): BatchScheduler's text_timeout)
+        self._text_feed = None  # text_stream.TextFeed, made and used by the scheduler thread
 
     def cancel(self):
         self.cancelled = True
+        if self._wake is not None:
+            self._wake.set()
+
+    def push_text(self, piece: str):
+        """Add a piece of an open request's text (thread-safe); the scheduler commits its tokens before its next launch."""
+        if not self.request.text_open:
+            raise ValueError("push_text: the request's text is not open (TTSRequest(text_open=True))")
+        with self._text_lock:
+            if self._text_closed:
+                raise ValueError("push_text after close_text")
+            self._pieces.append(str(piece))
+            self._t_text = time.monotonic()
+        if self._wake is not None:
+            self._wake.set()
+
+    def close_text(self):
+        """End an open request's text (thread-safe; a second call does nothing)."""
+        if not self.request.text_open:
+            raise ValueError("close_text: the request's text is not open (TTSRequest(text_open=True))")
+        with self._text_lock:
+            self._text_closed = True
+            self._t_text = time.monotonic()
+        if self._wake is not None:
+            self._wake.set()
+
+    def _take_text(self) -> Tuple[List[str], bool, float]:
+        """(pieces since the last call, text closed?, when text last arrived)."""
+        with self._text_lock:
+            pieces, self._pieces = self._pieces, []
+            return pieces, self._text_closed, self._t_text
 
     def chunks(self, timeout: Optional[float] = None) -> Iterator[Tuple[np.ndarray, int, dict]]:
         """The utterance's chunks as they arrive; `timeout` (seconds, for the whole utterance) raises TimeoutError and cancels
@@ -125,6 +168,11 @@ class _Active:
     emitted: int = 0
     budget: int = 0
     chunk_index: int = 0
+    open_text: bool = False  # TTSRequest(text_open=True): its text rows are appended before each launch
+    text_sent: int = 0       # committed text ids already in the slot (the first one is in the prompt)
+    talker: object = None    # text projection of the open text's rows
+    waiting: bool = False    # the stream waits for text (status.done = 4)
+    gen_step: int = 0
 
 
 class _StatefulAudio:
@@ -143,7 +191,7 @@ class BatchScheduler:
 
     def __init__(self, tts, chunk_frames: int = 8, max_concurrent: Optional[int] = None, seed: int = 0, codec_lanes: int = 4,
                  codec_mode: str = "auto", codec_split_k: Optional[bool] = None, overlap_codec="auto",
-                 emit_every: int = 1, mixed_policies: bool = False):
+                 emit_every: int = 1, mixed_policies: bool = False, text_timeout: float = 30.0):
         """codec_mode: "windowed" (default, = "auto") — the reference's 25-frame left-context re-decode (model.py:737-826): the
         audio is bit for bit what the single-stream streaming API returns for the same codes; "stateful" — one
         codec.CodecStream per slot: a chunk costs its own frames and the audio is the full non-streaming decode of the
@@ -166,7 +214,9 @@ class BatchScheduler:
         mixed_policies: no cohorts — requests take free slots first come, first served whatever their sampling policy; each
         admitted request's policy and seed (`TTSRequest.seed`, or one derived from `seed` and the request id) become its slot's
         own policy before its prefill, and every launch passes one fixed launch-wide policy that no live stream uses.  Off by
-        default: then a request that carries a `seed` is refused (the cohort shares the scheduler's `seed`)."""
+        default: then a request that carries a `seed` is refused (the cohort shares the scheduler's `seed`).
+        text_timeout: an open request (TTSRequest(text_open=True)) whose text has not ended and that receives no text for this many
+        seconds is cancelled (finish_reason "text_timeout"), so a slow client does not hold a slot for ever."""
         self.tts = tts
         self.emit_every = max(1, int(emit_every))
         self.codec_lanes = max(1, int(codec_lanes))
@@ -189,6 +239,7 @@ class BatchScheduler:
         self.max_concurrent = min(cap, max_concurrent or cap)
         self.seed = seed
         self.mixed_policies = bool(mixed_policies)
+        self.text_timeout = float(text_timeout)
         self._pending: "queue.Queue[RequestHandle]" = queue.Queue()
         self._deferred: List[RequestHandle] = []   # waiting for the running cohort's policy to drain
         self._active: Dict[int, _Active] = {}
@@ -245,30 +296,37 @@ class BatchScheduler:
         elif req.seed is not None:
             raise ValueError("a per-request seed needs BatchScheduler(mixed_policies=True): "
                              "in cohort mode the requests of a launch share the scheduler's seed")
+        if req.text_open and req.kind == "voice_clone" and not req.xvec_only:
+            raise ValueError("open text: an ICL voice clone sums the text into the reference-code rows; use xvec_only=True")
+        if req.text_open and req.kind == "voice_clone" and req.non_streaming_mode:
+            raise ValueError("open text needs non_streaming_mode=False (the whole text is in the prompt otherwise)")
         with self._submit_lock:
             h = RequestHandle(req, self._next_id)
             self._next_id += 1
         h._sr = self.tts.sample_rate
+        h._wake = self._wake
         self._pending.put(h)
         self._wake.set()
         return h
 
     # ---- scheduler thread ----
-    def _prepare(self, r: TTSRequest):
-        """Prompt embeddings exactly as the matching generate_* method builds them (model.py:202-330)."""
+    def _prepare(self, r: TTSRequest, text: Optional[str] = None):
+        """Prompt embeddings exactly as the matching generate_* method builds them (model.py:202-330); `text`: the text received
+        so far of an open request."""
         t = self.tts
+        text = r.text if text is None else text
         if r.kind == "voice_clone":
             m, _, _, tie, tam, tth, tpe, ref_codes = t._prepare_generation(
-                r.text, r.ref_audio, r.ref_text, language=r.language, xvec_only=r.xvec_only,
+                text, r.ref_audio, r.ref_text, language=r.language, xvec_only=r.xvec_only,
                 non_streaming_mode=r.non_streaming_mode, append_silence=r.append_silence, instruct=r.instruct)
             return m, tie, tam, tth, tpe, ref_codes
         if r.kind == "custom_voice":
             t._check_custom(r.language, r.speaker)
             instruct = None if t.model.model.tts_model_size in "0b6" else r.instruct  # model.py:849-850
-            m, _, _, tie, tam, tth, tpe = t._prepare_generation_custom(r.text, r.language, r.speaker, instruct)
+            m, _, _, tie, tam, tth, tpe = t._prepare_generation_custom(text, r.language, r.speaker, instruct)
         else:
             t._check_design(r.language)
-            m, _, _, tie, tam, tth, tpe = t._prepare_generation_custom(r.text, r.language, None, r.instruct)
+            m, _, _, tie, tam, tth, tpe = t._prepare_generation_custom(text, r.language, None, r.instruct)
         return m, tie, tam, tth, tpe, None
 
     def _policy(self, key: tuple, seed: Optional[int] = None) -> SamplingPolicy:
@@ -317,6 +375,19 @@ class BatchScheduler:
             if h.cancelled:
                 self._finish(h, "cancelled")
                 continue
+            if h.request.text_open:  # admitted once its first text token is committed; until then it holds no place in line
+                try:
+                    timed_out = self._pull_text(h)
+                except ValueError as e:  # e.g. the text closed empty
+                    h.q.put(e)
+                    self._finish(h, "error")
+                    continue
+                if not h._text_feed.ids:
+                    if timed_out:
+                        self._finish(h, "text_timeout")
+                    else:
+                        self._deferred.append(h)
+                    continue
             key = h.request.policy_key()
             if self.mixed_policies:
                 self._cohort = key  # no cohorts: whatever the policy, the request only waits for a free slot
@@ -328,13 +399,17 @@ class BatchScheduler:
                 self._deferred.append(h)
                 continue
             slot = free[0]
+            feed = h._text_feed
             try:
-                m, tie, tam, tth, tpe, ref_codes = self._prepare(h.request)
+                m, tie, tam, tth, tpe, ref_codes = self._prepare(h.request, None if feed is None else feed.text)
                 if tie.shape[1] > self.eng.max_seq_len:
                     raise RuntimeError(  # talker_graph.py:163-167
                         f"Input is too long: prefill has {tie.shape[1]} tokens but max_seq_len={self.eng.max_seq_len}. "
                         "Use shorter text or shorter reference audio.")
-                self.eng.set_text_conditioning(slot, tth[0], tpe)
+                if feed is None:
+                    self.eng.set_text_conditioning(slot, tth[0], tpe)
+                else:  # the prompt holds the first text token; the rest arrive as trailing rows (text_stream.py)
+                    self.eng.open_text(slot, tpe)
                 if self.mixed_policies:
                     self.eng.set_stream_policy(slot, self._policy(key, self.request_seed(h)))
                     self.eng.prefill(slot, tie[0], _left_pads(tam), self._launch_policy())
@@ -360,8 +435,59 @@ class BatchScheduler:
                 window = _StatefulAudio(cs, lane_tok.sample_rate)
             else:
                 window = WindowedDecode(lane_tok, ref_codes, self.chunk_frames)
-            self._active[slot] = _Active(h, slot, window, budget=min(h.request.max_new_tokens, self.eng.max_frames))
+            a = self._active[slot] = _Active(h, slot, window, budget=min(h.request.max_new_tokens, self.eng.max_frames))
+            if feed is not None:
+                a.open_text, a.talker, a.text_sent, a.waiting = True, m.talker, 1, True  # prefilled without a second token
+                self._append_text(a)
             self.stats["requests"] += 1
+
+    def _pull_text(self, h: RequestHandle) -> bool:
+        """Commit the pieces an open request received since the last call (text_stream.TextFeed); returns whether its text
+        has been silent for text_timeout seconds without being closed."""
+        from .text_stream import TextFeed
+
+        if h._text_feed is None:
+            h._text_feed = TextFeed(self.tts.model.tokenizer.assistant, self.tts.model.model.config.tts_eos_token_id)
+        pieces, closed, t_text = h._take_text()
+        for p in pieces:
+            h._text_feed.push(p)
+        if closed:
+            h._text_feed.close()
+        return not closed and time.monotonic() - t_text > self.text_timeout
+
+    def _append_text(self, a: _Active):
+        """The committed text of an open slot that is not on the device yet (and the close)."""
+        from .text_stream import text_rows
+
+        feed = a.handle._text_feed
+        new = feed.ids[a.text_sent:]
+        if new:  # a close always commits the tts_eos id, so it travels with rows
+            self.eng.append_text(a.slot, text_rows(a.talker, new), close=feed.closed)
+            a.text_sent = len(feed.ids)
+        rows = a.text_sent - 1  # trailing rows: the first committed token is in the prompt
+        a.waiting = a.waiting and not (feed.closed or rows > a.gen_step)
+
+    def _service_open(self):
+        """Before a launch: append what every open slot received; cancel a cancelled or silent one (its slot is free again)."""
+        for slot in sorted(self._active):
+            a = self._active[slot]
+            if not a.open_text:
+                continue
+            reason = "cancelled" if a.handle.cancelled else None
+            if reason is None:
+                try:
+                    timed_out = self._pull_text(a.handle)
+                except ValueError as e:
+                    a.handle.q.put(e)
+                    timed_out, reason = False, "error"
+                if timed_out:
+                    reason = "text_timeout"
+                elif reason is None:
+                    self._append_text(a)
+            if reason is not None:
+                self._finish(a.handle, reason)
+                self._release(slot)
+                del self._active[slot]
 
     def _finish(self, h: RequestHandle, reason: str):
         h.finish_reason = reason
@@ -453,8 +579,15 @@ class BatchScheduler:
                 while not self._stop.is_set():
                     t0 = time.perf_counter()
                     self._admit()
+                    self._service_open()
                     t1 = time.perf_counter()
                     self.stats["t_admit"] += t1 - t0
+                    if self._active and all(a.waiting for a in self._active.values()):
+                        self._emit(self._backlog)  # every running stream waits for text: no launch until some arrives
+                        self._backlog = []
+                        self._wake.wait(timeout=0.05)
+                        self._wake.clear()
+                        continue
                     if not self._active:
                         self._emit(self._backlog)
                         self._backlog = []
@@ -495,6 +628,8 @@ class BatchScheduler:
                         st = eng.status(slot)  # synchronises the launch (first call) and reads the slot's counters
                         if st.error:
                             raise RuntimeError(f"device fault {st.error} in slot {slot}")
+                        if a.open_text:
+                            a.waiting, a.gen_step = st.done == 4, st.gen_step
                         n_new = min(st.n_frames, a.budget) - a.emitted
                         reason = None
                         if a.handle.cancelled:
@@ -508,6 +643,8 @@ class BatchScheduler:
                         if n_new > 0 and reason is None and a.emitted > 0 and n_new < self.emit_every * self.chunk_frames:
                             # emit_every > 1: after an utterance's first chunk, hand audio out every few chunks
                             continue
+                        if reason is None:  # whole chunks only (a stream that waited for text ran part of one)
+                            n_new -= n_new % self.chunk_frames
                         if n_new > 0 and reason != "cancelled":
                             chunk = eng.read_codes(slot, a.emitted, n_new)
                             a.emitted += n_new
