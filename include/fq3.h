@@ -236,6 +236,18 @@ int fq3_debug_set_epoch(fq3_engine* e, uint32_t epoch);
  * `stream_idx`'s last talker sampling phase consumed.  Valid right after an fq3_decode_frames launch of the
  * reference-shaped program (not the wide one) that ran the stream; -FQ3_E_INVALID otherwise. */
 int fq3_debug_read_talker_logits(fq3_engine* e, int stream_idx, void* out_f32, void* stream);
+/* Test hook: the LAST talker layer's fused q|k|v projection row (bf16 [(nq + 2*nkv) * 128]: raw q_proj | k_proj | v_proj
+ * outputs, before q/k RMSNorm and RoPE) and its attention output row (bf16 [nq * 128], before o_proj) for activation row
+ * `row` of the last persistent launch that ran the talker.  Rows of each launch kind:
+ *   fq3_talker_step: 0;
+ *   fq3_prefill / fq3_prefill_tail: the row within the LAST chunk of the prompt; chunks start at the first row the call
+ *     computes (0, or T - n_tail) and take as many rows as fit (at most 8), so row r is position T - n_last + r where n_last
+ *     is the size of the last chunk;
+ *   fq3_decode_frames: the stream's index within the last launched lock-step group (row r is the group's first stream + r),
+ *     in the reference-shaped and the wide program alike, for the last frame of the launch.
+ * fq3_prefill_head and fq3_predictor_run do not run the talker's layers and leave the rows of the launch before them.
+ * -FQ3_E_INVALID for a row the last launch that ran the talker did not run. */
+int fq3_debug_read_talker_attn(fq3_engine* e, int row, void* out_qkv_bf16, void* out_attn_bf16, void* stream);
 /* Copy status / codes back (synchronises `stream`). codes_out: host int32 [n, 16]. */
 int fq3_get_status(fq3_engine* e, int stream_idx, fq3_status* out, void* stream);
 int fq3_read_codes(fq3_engine* e, int stream_idx, int first_frame, int n, int32_t* codes_out, void* stream);

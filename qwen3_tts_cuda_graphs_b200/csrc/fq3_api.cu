@@ -64,6 +64,7 @@ struct fq3_engine {
   int* err_dev = nullptr;
   float* pred_logits_all = nullptr;
   int frames_rows = 0;  // streams of the last persistent launch if it ran the reference-shaped frame program, else 0
+  int talker_rows = 0;  // activation rows of the last persistent launch that ran the talker's layers (fq3_debug_read_talker_attn)
   uint8_t* seen_scratch = nullptr;
   Phase *d_frames = nullptr, *d_pred = nullptr, *d_talker = nullptr, *d_prefill = nullptr, *d_linear = nullptr, *d_wide = nullptr;
   std::vector<Phase> h_frames, h_pred, h_talker, h_prefill, h_wide;  // host copies (shared-memory sizing)
@@ -446,6 +447,11 @@ int launch(fq3_engine* e, LaunchParams& p, const Phase* prog_host, cudaStream_t 
   CK(cudaLaunchCooperativeKernel(fn, dim3(grid), dim3(kThreads), args, smem, s));
   e->launches += 1;
   e->frames_rows = (p.mode == MODE_FRAMES && !p.wide) ? p.n_rows : 0;
+  for (int i = 0; i < p.n_phases; ++i)
+    if (prog_host[i].type == PH_ATTN && prog_host[i].stack == ST_TALKER) {
+      e->talker_rows = p.n_rows;  // talker row r of every launch kind is activation row r (kernel: get_group)
+      break;
+    }
   return 0;
 }
 
@@ -1180,6 +1186,16 @@ int fq3_debug_read_talker_logits(fq3_engine* e, int idx, void* out_f32, void* st
   if (idx >= e->frames_rows)
     return fail(FQ3_E_INVALID, "the last launch was not a reference-shaped fq3_decode_frames launch that ran this stream");
   return unpack_f32(e, out_f32, e->tk.d.vocab, BUF_LOGITS, idx, 1, e->tk.d.vocab, (cudaStream_t)stream);
+}
+
+// Nothing after the talker's last layer writes BUF_TQKV / BUF_TATT, so until the next launch that runs the talker they hold
+// that layer's rows.
+int fq3_debug_read_talker_attn(fq3_engine* e, int row, void* out_qkv_bf16, void* out_attn_bf16, void* stream) {
+  if (!e || !out_qkv_bf16 || !out_attn_bf16) return fail(FQ3_E_INVALID, "bad arguments");
+  if (row < 0 || row >= e->talker_rows) return fail(FQ3_E_INVALID, "the last launch that ran the talker did not run this row");
+  const cudaStream_t s = (cudaStream_t)stream;
+  if (int r = unpack_bf16(e, out_qkv_bf16, e->tk.qkvdim(), BUF_TQKV, row, 1, e->tk.qkvdim(), s)) return r;
+  return unpack_bf16(e, out_attn_bf16, e->tk.qdim(), BUF_TATT, row, 1, e->tk.qdim(), s);
 }
 
 int fq3_get_status(fq3_engine* e, int idx, fq3_status* out, void* stream) {

@@ -305,6 +305,15 @@ class Engine:
         _lib.check(self.lib.fq3_debug_read_talker_logits(self.h, int(idx), out.data_ptr(), _stream()))
         return out
 
+    def debug_talker_attn(self, row: int = 0):
+        """(qkv bf16 [(nq + 2 nkv) * 128], attn bf16 [nq * 128]): the last talker layer's raw fused q|k|v projection and attention
+        output of activation row `row` of the last launch that ran the talker (fq3.h test hook, row mapping there)."""
+        t = self.cfg.talker
+        qkv = torch.empty((t.num_attention_heads + 2 * t.num_key_value_heads) * t.head_dim, dtype=torch.bfloat16, device=self.device)
+        attn = torch.empty(t.num_attention_heads * t.head_dim, dtype=torch.bfloat16, device=self.device)
+        _lib.check(self.lib.fq3_debug_read_talker_attn(self.h, int(row), qkv.data_ptr(), attn.data_ptr(), _stream()))
+        return qkv, attn
+
     def last_hidden(self, row: int = 0) -> torch.Tensor:
         out = torch.empty(self.cfg.talker.hidden_size, dtype=torch.bfloat16, device=self.device)
         _lib.check(self.lib.fq3_last_hidden(self.h, int(row), out.data_ptr(), _stream()))

@@ -192,21 +192,24 @@ def test_predictor_matches_oracle_teacher_forced(pair):
 def test_frame_loop_teacher_forced_against_oracle(pair):
     """Every id the device loop emits must be the oracle's greedy choice at that step, up to bf16 near-ties."""
     cfg, w, eng, orc = pair
-    tie, tam, tth, tpe = synth_prompt(cfg, T=14, R=3)
+    _frame_loop_teacher_forced(cfg, eng, orc, T=14, n=10)
+
+
+def _frame_loop_teacher_forced(cfg, eng, orc, T, n):
+    tie, tam, tth, tpe = synth_prompt(cfg, T=T, R=3)
     pol = _sp(do_sample=False, repetition_penalty=1.05, min_new_tokens=2)
-    n = 10
     eng.set_text_conditioning(0, tth[0].cuda(), tpe.cuda())
     eng.prefill(0, tie[0].cuda(), 0, pol)
     tok0 = eng.status(0).token
     eng.decode_frames(1, n, pol, _sub(do_sample=False))
     st = eng.status(0)
-    assert st.error == 0 and st.n_frames == n and st.position == 14 + n and st.gen_step == n
+    assert st.error == 0 and st.n_frames == n and st.position == T + n and st.gen_step == n
     codes = eng.read_codes(0, 0, n)
     assert codes[0, 0] == tok0
     orc.sub.do_sample = False
     trace = {}
     frames = list(orc.generate_frames(tie, tam, tth, tpe, max_new_tokens=n, min_new_tokens=2, do_sample=False,
-                                      repetition_penalty=1.05, max_seq_len=272, trace=trace, forced=codes))
+                                      repetition_penalty=1.05, max_seq_len=eng.max_seq_len, trace=trace, forced=codes))
     assert len(frames) == n
     bad = []
     tscale = float(trace["prefill_logits"].abs().max())
@@ -412,6 +415,15 @@ def test_wide_streams_match_single_stream_real_dims():
     _batch_vs_single(cfg, w, 16, 8, lens=[14, 60, 37, 101])
 
 
+def test_wide_streams_match_single_stream_past_768():
+    """0.6B dims, two layers, 16 streams with contexts on both sides of 768 positions: past 768 a split holds more than 48
+    positions (the long-range path) and the wide program's attention leaves its one-item-per-stream path for the generic walk,
+    which mixes the short streams' items with the long streams' split items in one launch."""
+    cfg = make_cfg("0.6B-Base", 2, 2)
+    w = make_weights(cfg, seed=0)
+    _batch_vs_single(cfg, w, 16, 4, lens=[700, 768, 769, 1500], max_seq_len=2048)
+
+
 def test_wide_streams_match_single_stream_full_depth():
     """The real 0.6B stack at full depth (28 + 5 layers), 16 streams with contexts from 14 to 201 positions (one to five KV
     splits): 8 frames of every stream equal its single-stream run."""
@@ -509,14 +521,17 @@ def test_first_token_sampler_respects_suppression_and_top_k(tiny):
 # ------------------------------------------------------------------------------------------------
 # dense (tcgen05) prefill against the chunked decode-kernel prefill
 # ------------------------------------------------------------------------------------------------
-@pytest.mark.parametrize("T", [17, 40, 130, 240])
-def test_dense_prefill_matches_chunked_prefill(pair, T, monkeypatch):
+@pytest.mark.parametrize("T", [17, 40, 130, 240, 2047])
+def test_dense_prefill_matches_chunked_prefill(pair, T, monkeypatch, request):
     """The tensor-core prefill must give the logits and the first token of the all-decode-kernel prefill, and the K/V it wrote
     must serve the next decode step (hidden state vs the oracle) — in both of its forms: all T rows through all layers +
-    fq3_prefill_head (default), and rows [0, T-1) + the last row through the decode kernel (fq3_prefill_tail, FQ3_DENSE_FULL=0)."""
+    fq3_prefill_head (default), and rows [0, T-1) + the last row through the decode kernel (fq3_prefill_tail, FQ3_DENSE_FULL=0).
+    T = 2047 (fq3c_attn_prefill_kernel takes M <= 2048) runs on the tiny preset's 2048-position engine."""
     cfg, w, eng, orc = pair
     if T >= eng.max_seq_len:
-        pytest.skip("prompt longer than this fixture's cache")
+        if cfg.talker.num_key_value_heads != 2:
+            pytest.skip("prompt longer than this fixture's cache")
+        cfg, w, eng, orc = request.getfixturevalue("long_pair")
     tie, tam, tth, tpe = synth_prompt(cfg, T=T, seed=5)
     pol = _sp(do_sample=False, repetition_penalty=1.0, min_new_tokens=2)
     xg = (0.05 * torch.randn(1, 1, cfg.talker.hidden_size, generator=torch.Generator().manual_seed(9))).to(torch.bfloat16)
@@ -581,23 +596,25 @@ def test_dense_prefill_fused_row_norm_is_bit_identical(pair, T, monkeypatch):
 
 
 # ------------------------------------------------------------------------------------------------
-# long contexts: split-KV attention (48 positions per CTA) with the combine step, up to ten splits
+# long contexts: split-KV attention (48 positions per CTA) with the combine step, up to 16 splits; beyond 768 positions a
+# split holds more than 48 (the half-warp online-softmax path)
 # ------------------------------------------------------------------------------------------------
 @pytest.fixture(scope="module")
 def long_pair():
     name, tl, pl = CONFIGS[0]
     cfg = make_cfg(name, tl, pl)
     w = make_weights(cfg, seed=13)
-    eng = make_engine(cfg, w, max_seq_len=512)
+    eng = make_engine(cfg, w, max_seq_len=2048)
     orc = make_oracle(cfg, w)
     yield cfg, w, eng, orc
     eng.close()
 
 
-@pytest.mark.parametrize("T", [49, 97, 150, 192, 193, 300, 470])
+@pytest.mark.parametrize("T", [49, 97, 150, 192, 193, 300, 470, 760, 767, 768, 1200, 2046])
 def test_talker_step_long_context_matches_oracle(long_pair, T):
-    """A decode step at position T attends to T+1 positions: one CTA per (kv head, split of <= 48 positions) and the combine
-    step of split 0, for 2 to 10 splits (three combine rounds).  Hidden state and the prefill logits against the oracle."""
+    """A decode step at position T attends to T+1 positions: one CTA per (kv head, split) and the combine step of split 0, for
+    2 to 16 splits (four combine rounds), splits of more than 48 positions from T = 768 on.  Hidden state and the prefill logits
+    against the oracle."""
     cfg, w, eng, orc = long_pair
     tie, tam, tth, tpe = synth_prompt(cfg, T=T, seed=100 + T)
     pol = _sp(do_sample=False, repetition_penalty=1.0, min_new_tokens=2)
@@ -614,3 +631,10 @@ def test_talker_step_long_context_matches_oracle(long_pair, T):
         torch.cuda.synchronize()
         assert eng.status(0).error == 0
         assert rel_err(h, ref_h) <= TOL, (step, rel_err(h, ref_h))
+
+
+def test_frame_loop_teacher_forced_across_768(long_pair):
+    """A 760-row prompt and 16 greedy frames: the talker's context runs from 761 to 776 positions, so the frame loop moves from
+    the two-pass split path to the long-range path mid-stream."""
+    cfg, w, eng, orc = long_pair
+    _frame_loop_teacher_forced(cfg, eng, orc, T=760, n=16)
